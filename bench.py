@@ -1,6 +1,6 @@
 """Contract benchmark: poses/sec of the Gen6D inference hot path (detect -> select -> 3x refine).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pose: a synthetic 480x640 frame through the detector (32 reference views,
 4 scales), the 128x128 crop through the selector (64 reference views x 5 in-plane angles), and
@@ -15,8 +15,11 @@ three refinement iterations (6 views, 32^3 volume) -- BASELINE.json's full-estim
 
 N > 1 (torchrun): one process per GPU, each rank runs an independent replica on its own frames
 (weak scaling, no data-path collective; poses are all-gathered once at the end over NCCL).
-`--impl reference` times the CPU oracle port instead (the reference itself cannot travel to the
-GPU box: /root/reference does not exist there).
+`--impl reference` times the CPU oracle port instead (the reference itself is not part of this
+repository).
+`--dump-outputs DIR` writes, after the timed steps, what the device-resident path computed for its last
+batch and the poses the timed end-to-end call returned (see write_outputs); the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -333,6 +336,45 @@ def run_reference_arm(args, rank, world):
     print(json.dumps(line))
 
 
+DUMP_LIMIT = 64 << 20           # bytes of .npy files --dump-outputs may write
+DUMP_SEED = 0
+STAGE_OUTPUTS = {'predict': ('poses', 'detection', 'crop', 'ref_idx', 'selection', 'logits')}   # Gen6DEstimator._predict_device_fn
+
+
+def stage_outputs(outs):
+    """[(stage name, tensor or tuple of tensors)] of one batch -> {'<stage>.<output>': host array}.  A stage name that
+    recurs (the per-iteration refine stages of the host-sequenced path) gets its occurrence number appended."""
+    names = [n for n, _ in outs]
+    seen, res = {}, {}
+    for name, o in outs:
+        seen[name] = seen.get(name, 0) + 1
+        stage = name if names.count(name) == 1 else f'{name}{seen[name] - 1}'
+        o = o if isinstance(o, (tuple, list)) else (o,)
+        labels = STAGE_OUTPUTS.get(name, ())
+        for j, t in enumerate(o):
+            res[f'{stage}.{labels[j] if j < len(labels) else j}'] = t.detach().cpu().numpy()
+    return res
+
+
+def write_outputs(path, arrays, limit=DUMP_LIMIT):
+    """Writes every array as path/<name>.npy: floating point as float32 (float64 stays float64), integers as float64
+    (exact).  An array above its equal share of `limit` is replaced by a fixed, seeded sample of its flattened
+    elements, in order.  Returns {name: [shape written, shape computed]}."""
+    os.makedirs(path, exist_ok=True)
+    share = (limit - 256 * len(arrays)) // max(1, len(arrays))      # 256 bytes of .npy header per file at most
+    written = {}
+    for name, a in sorted(arrays.items()):
+        a = np.asarray(a)
+        full = list(a.shape)
+        a = a.astype(np.float64 if a.dtype == np.float64 or a.dtype.kind in 'biu' else np.float32)
+        if a.nbytes > share:
+            keep = np.random.default_rng(DUMP_SEED).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(keep)]
+        np.save(os.path.join(path, name + '.npy'), a)
+        written[name] = [list(a.shape), full]
+    return written
+
+
 # ---------------------------------------------------------------------------------------------
 def run_ours(args, rank, world, local_rank):
     from gen6d_b200 import _lib, graphs, ops
@@ -363,9 +405,10 @@ def run_ours(args, rank, world, local_rank):
     # host geometry and copies.  W lanes (clones with private graphs, shared weights / reference features),
     # each on its own stream, keep W x B frames in flight.
     W, Bt = E2E_WORKERS, pick_batch(args.steps, E2E_WORKERS)
+    tail = args.steps % Bt          # poses of the short last batch of the timed region
     batch_imgs = [db.get_image(frames[i % len(frames)]) for i in range(Bt)]
 
-    def record(e):
+    def record(e, n):
         rec, mods = [], [m for m in (e, e.detector, e.selector, e.refiner) if m is not None]     # e: the whole-prediction graph (device_glue)
         for m in mods:
             def wrapped(name, fn, inputs, _m=m, _o=m.stages.run):
@@ -373,38 +416,44 @@ def run_ours(args, rank, world, local_rank):
                 return _o(name, fn, inputs)
             m.stages.run = wrapped
         try:
-            e.predict_batch(batch_imgs, [K] * Bt)
+            e.predict_batch(batch_imgs[:n], [K] * n)
         finally:
             for m in mods:
                 del m.stages.run
         return rec
 
     lanes = [torch.cuda.Stream() for _ in range(W)]
-    recs = []
+    recs, recs_tail = [], []
     for i in range(W):
         e = est if i == 0 else est.worker_clone()
         with torch.cuda.stream(lanes[i]):
-            recs.append(record(e))
+            recs.append(record(e, Bt))
+            if tail:
+                recs_tail.append(record(e, tail))
             lanes[i].synchronize()
     det, sel, rfr = est.detector, est.selector, est.refiner
 
-    def device_batch(i=0, eager=False):
-        """One batch of Bt poses on lane i through the captured stage graphs (eager=True: kernel by kernel)."""
+    def device_batch(i=0, eager=False, short=False):
+        """One batch of Bt poses (short=True: of `tail` poses) on lane i through the captured stage graphs (eager=True:
+        kernel by kernel).  Returns [(stage name, outputs)] in launch order."""
+        outs = []
         with torch.no_grad():
-            for m, name, fn, inputs in recs[0 if eager else i % W]:
-                if eager:
-                    fn(*inputs)
-                else:
-                    m.stages.run(name, fn, inputs)
+            for m, name, fn, inputs in (recs_tail if short else recs)[0 if eager else i % W]:
+                outs.append((name, fn(*inputs) if eager else m.stages.run(name, fn, inputs)))
+        return outs
+
+    last_outputs = []
 
     def device_steps(n):
-        """n poses = ceil(n / Bt) batches dealt round-robin to the lanes (a short last batch runs full)."""
+        """n poses = n // Bt full batches and, for n % Bt == tail, one short batch, dealt round-robin to the lanes."""
+        nb, short = divmod(n, Bt)
+        assert short in (0, tail), (n, Bt, tail)
         main = torch.cuda.current_stream()
         for st in lanes:
             st.wait_stream(main)
-        for i in range((n + Bt - 1) // Bt):
+        for i in range(nb + (short > 0)):
             with torch.cuda.stream(lanes[i % W]):
-                device_batch(i)
+                last_outputs[:] = device_batch(i, short=i == nb)
         for st in lanes:
             main.wait_stream(st)
 
@@ -446,7 +495,8 @@ def run_ours(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     note('stage graphs recorded')
-    dev_ms, _, launches = timed(device_steps, args.steps, max(args.warmup, 2 * W * Bt), batched=True)
+    dev_ms, _, launches = timed(device_steps, args.steps, -(-max(args.warmup, 2 * W * Bt) // Bt) * Bt, batched=True)
+    dumps = stage_outputs(last_outputs) if args.dump_outputs else {}
 
     note('device-resident timing done')
     # ---- end to end through the public API (numpy in, numpy out)
@@ -475,6 +525,8 @@ def run_ours(args, rank, world, local_rank):
     pipelined(args.steps)
     torch.cuda.synchronize()
     pipe_ms = (time.perf_counter() - t0) * 1e3
+    if args.dump_outputs:
+        dumps['e2e.poses'] = np.stack(out_poses[-args.steps:], 0)
     barrier()
     if world > 1:
         import torch.distributed as dist
@@ -567,6 +619,8 @@ def run_ours(args, rank, world, local_rank):
         line['accuracy'] = accuracy
     if sharded is not None:
         line['sharded'] = sharded
+    if args.dump_outputs:
+        line['dumped_outputs'] = write_outputs(args.dump_outputs, dumps)
     if world == 1:
         try:
             line['torch_cuda_baseline'] = torch_cuda_baseline(5, 2)
@@ -591,7 +645,12 @@ def main():
     ap.add_argument('--steps', type=int, default=None)
     ap.add_argument('--warmup', type=int, default=None)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference', 'torch-cuda'])
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the timed device-resident path computed in its last batch, and the poses of the timed '
+                         'end-to-end call, as DIR/<name>.npy (float32 / float64, at most 64 MB in all)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     rank, world = int(os.environ.get('RANK', 0)), int(os.environ.get('WORLD_SIZE', 1))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
     if args.impl == 'reference':
