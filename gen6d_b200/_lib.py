@@ -60,6 +60,8 @@ _SIGNATURES = {
     'g6d_glue_refine_problems_host': [C.POINTER(GlueViews), P, P, I, I, P, I, I, P, P, P, P, P, P, P],
     'g6d_glue_apply_refinements': [C.POINTER(GlueViews), P, P, P, P, I, P, P],
     'g6d_glue_apply_refinements_host': [C.POINTER(GlueViews), P, P, P, P, I, P],
+    'g6d_track_smooth': [P, P, P, P, P, I, I, P, P, P, P, P, P],
+    'g6d_track_smooth_host': [P, P, P, P, P, I, I, P, P, P, P, P],
     'g6d_nchw_to_nhwc': [P, P, I, I, I, I, I, P],
     'g6d_nhwc_to_nchw': [P, P, I, I, I, I, I, P],
     'g6d_resize_bilinear': [P, P, I, I, I, I, I, I, I, I, P],

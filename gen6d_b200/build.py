@@ -11,7 +11,7 @@ LIB = os.path.join(HERE, 'libgen6d_b200.so')
 STAMP = os.path.join(HERE, '.libgen6d_b200.hash')
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-Xcompiler', '-fPIC']
-NO_FMA = ('glue.cu',)
+NO_FMA = ('glue.cu', 'track.cu')
 
 
 def sources():

@@ -218,7 +218,11 @@ class Gen6DEstimator:
         with torch.no_grad():
             cams = self.detector._to_dev(glue.cameras(np.stack(que_Ks, 0)))
             outs = self.stages.run('predict', self._predict_device_fn(st), [frames, cams])
-            chain, det, crop, idx, sel_out, logits = [self.detector._to_host(t) for t in outs]
+            return self._device_results(outs, qn)
+
+    def _device_results(self, outs, qn):
+        """_predict_device_fn's outputs -> predict_batch's (poses, inter), read back to the host."""
+        chain, det, crop, idx, sel_out, logits = [self.detector._to_host(t) for t in outs]
         chain = chain.reshape(len(chain), qn, 3, 4)
         poses0, refined = chain[0], [c.astype(np.float32) for c in chain[1:]]
         inter = {'det_position': det[:, :2].copy(), 'det_scale_r2q': det[:, 2].copy(), 'det_que_img': crop,

@@ -137,3 +137,43 @@ def host_apply_refinements(tables, prob, net_out):
                                                           prob['pose_rect'].ctypes.data, net.ctypes.data, len(net), poses.ctypes.data),
                'g6d_glue_apply_refinements_host')
     return poses
+
+
+# ------------------------------------------------------------------------------------------ pose smoothing (csrc/track.cu)
+def smoothing_weights(num, std):
+    """predict.py:19-23: weights = exp(-(arange(num) / std) ** 2)[::-1] (newest last, weight 1) and wsum[n - 1] = the sum
+    of the last n of them, the normaliser of a history of n < num projections -- both evaluated by numpy, so that the
+    kernel's average divides by exactly what the reference divides by."""
+    w = np.ascontiguousarray(np.exp(-(np.arange(num) / std) ** 2)[::-1], np.float64)
+    return w, np.asarray([np.sum(w[-n:]) for n in range(1, num + 1)], np.float64)
+
+
+def check_bbox(bbox_3d):
+    """bbox_3d -> float32 [8,3]; ValueError unless it is 8 x 3 and non-coplanar by cv::solvePnP's test (the smallest over
+    the middle singular value of the centred points' 3x3 scatter matrix >= 1e-3; below it OpenCV takes its planar
+    homography branch, which the smoothing kernel does not implement)."""
+    b = np.asarray(bbox_3d)
+    if b.shape != (8, 3) or not np.all(np.isfinite(b)):
+        raise ValueError(f'bbox_3d must be 8 x 3 finite corners, got shape {b.shape}')
+    b = np.ascontiguousarray(b, np.float32)
+    c = b.astype(np.float64) - b.astype(np.float64).mean(0)
+    w = np.linalg.svd(c.T @ c, compute_uv=False)
+    if not w[1] > 0 or w[2] / w[1] < 1e-3:
+        raise ValueError('bbox_3d is degenerate or planar: the smoothing PnP needs non-coplanar corners')
+    return b
+
+
+def host_track_smooth(bbox, poses, cams, weights, wsum, hist, count):
+    """g6d_track_smooth_host: the kernel's code on numpy arrays.  hist f32 [M,num,8,2] and count i32 [M] are updated in
+    place.  Returns (corners f32 [M,8,2], averaged corners f64 [M,8,2], smoothed poses f64 [M,3,4])."""
+    bbox = np.ascontiguousarray(bbox, np.float32)
+    poses = np.ascontiguousarray(np.asarray(poses, np.float64).reshape(-1, 12))
+    cams = np.ascontiguousarray(cams, np.float64)
+    weights, wsum = np.ascontiguousarray(weights, np.float64), np.ascontiguousarray(wsum, np.float64)
+    assert hist.dtype == np.float32 and hist.flags.c_contiguous and count.dtype == np.int32 and count.flags.c_contiguous
+    M = len(poses)
+    corners, wpts, smoothed = np.zeros((M, 8, 2), np.float32), np.zeros((M, 8, 2), np.float64), np.zeros((M, 3, 4), np.float64)
+    _lib.check(_lib.lib().g6d_track_smooth_host(bbox.ctypes.data, poses.ctypes.data, cams.ctypes.data, weights.ctypes.data,
+                                                wsum.ctypes.data, M, len(weights), hist.ctypes.data, count.ctypes.data,
+                                                corners.ctypes.data, wpts.ctypes.data, smoothed.ctypes.data), 'g6d_track_smooth_host')
+    return corners, wpts, smoothed

@@ -21,10 +21,13 @@ def graphs_enabled():
 
 
 class CapturedStage:
-    """fn(*tensors) -> tensor or tuple of tensors, captured for one input-shape signature."""
+    """fn(*tensors) -> tensor or tuple of tensors, captured for one input-shape signature.  `state`: tensors that fn
+    updates in place and that carry over from call to call (a tracker's poses and history); the warm-up runs must not
+    advance them, so they are restored after the capture."""
 
-    def __init__(self, fn, example_inputs, warmup=2):
+    def __init__(self, fn, example_inputs, warmup=2, state=()):
         self.static_in = [t.clone() for t in example_inputs]
+        saved = [t.clone() for t in state]
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side), torch.no_grad():
@@ -38,6 +41,8 @@ class CapturedStage:
         with torch.cuda.graph(self.graph, capture_error_mode='thread_local'), torch.no_grad():
             self.static_out = fn(*self.static_in)
         self.kernels = _lib.launch_count() - before     # kernel nodes captured (our C-ABI launches)
+        for t, s in zip(state, saved):
+            t.copy_(s)
 
     def __call__(self, *inputs):
         for s, t in zip(self.static_in, inputs):
@@ -56,11 +61,11 @@ class StageCache:
     def clear(self):
         self.stages.clear()
 
-    def run(self, name, fn, inputs):
+    def run(self, name, fn, inputs, state=()):
         if not graphs_enabled():
             return fn(*inputs)
         key = (name,) + tuple((tuple(t.shape), t.dtype) for t in inputs)
         st = self.stages.get(key)
         if st is None:
-            st = self.stages[key] = CapturedStage(fn, inputs)
+            st = self.stages[key] = CapturedStage(fn, inputs, state=state)
         return st(*inputs)

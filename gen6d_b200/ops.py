@@ -142,6 +142,20 @@ def glue_apply_refinements(views_struct, que_pose, que_K, rect, net_out):
     return poses
 
 
+def track_smooth(bbox, poses, cams, weights, wsum, hist, count):
+    """One tracked frame of pose smoothing per lane (csrc/track.cu): bbox f32 [8,3], poses f64 [M,12], cams f64 [M,20],
+    weights / wsum f64 [num] (glue.smoothing_weights), history ring hist f32 [M,num,8,2] and count i32 [M] (updated in
+    place) -> (corners f32 [M,8,2], averaged corners f64 [M,8,2], smoothed poses f64 [M,12])."""
+    M, num = poses.shape[0], weights.shape[0]
+    corners = torch.empty(M, 8, 2, device=poses.device, dtype=torch.float32)
+    wpts = torch.empty(M, 8, 2, device=poses.device, dtype=torch.float64)
+    smoothed = torch.empty(M, 12, device=poses.device, dtype=torch.float64)
+    _call('g6d_track_smooth', _p(bbox), _p(poses, torch.float64), _p(cams, torch.float64), _p(weights, torch.float64),
+          _p(wsum, torch.float64), M, num, _p(hist), _p(count, torch.int32), _p(corners), _p(wpts, torch.float64),
+          _p(smoothed, torch.float64), _stream())
+    return corners, wpts, smoothed
+
+
 def imagenet_norm(x, out_c=4):
     out = torch.empty(*x.shape[:-1], out_c, device=x.device, dtype=torch.float32)
     _call('g6d_imagenet_norm', _p(x), _p(out), x.numel() // x.shape[-1], x.shape[-1], out_c, _stream())

@@ -122,6 +122,19 @@ int g6d_glue_apply_refinements(const g6d_glue_views* views, const float* que_pos
                                const float* net_out, int qn, double* poses, g6d_stream_t stream);
 int g6d_glue_apply_refinements_host(const g6d_glue_views* views, const float* que_pose, const float* que_K, const float* rect,
                                     const float* net_out, int qn, double* poses);
+
+/* ---- pose smoothing of a tracked video (predict.py:18-26, 63-71; utils/base_utils.py:256-265 project_points;
+ * utils/pose_utils.py:246-279 pnp).  One thread per lane (lanes <= 64): project the 8 box corners bbox [8,3] with the
+ * lane's pose (float64 storage of float32 values) and cams[lane].K in float32, push them into the lane's history ring
+ * hist [lanes,num,8,2] (float32) at slot count[lane] % num and increment count[lane], average the last min(count, num)
+ * entries with weights[num - n .. num) / wsum[n - 1] in float64, and solve SOLVEPNP_ITERATIVE (non-coplanar DLT + LM,
+ * float64) for the averaged points.  weights [num] = exp(-(arange(num) / std) ** 2)[::-1] and wsum[n - 1] = the numpy
+ * sum of its last n entries, both from the caller.  Outputs: corners [lanes,8,2] float32, wpts [lanes,8,2] float64,
+ * smoothed [lanes,12] float64 [R | t]. */
+int g6d_track_smooth(const float* bbox, const double* poses, const g6d_glue_camera* cams, const double* weights, const double* wsum,
+                     int lanes, int num, float* hist, int* count, float* corners, double* wpts, double* smoothed, g6d_stream_t stream);
+int g6d_track_smooth_host(const float* bbox, const double* poses, const g6d_glue_camera* cams, const double* weights, const double* wsum,
+                          int lanes, int num, float* hist, int* count, float* corners, double* wpts, double* smoothed);
 /* (x - mean) / std on f32 [n_pixels, in_c] -> [n_pixels, out_c] (in_c, out_c in {3,4})
  * (network/detector.py:189, selector.py:115, refiner.py:65) */
 int g6d_imagenet_norm(const float* in, float* out, long long n_pixels, int in_c, int out_c, g6d_stream_t stream);
