@@ -21,7 +21,8 @@ TC_TF32, TC_F16 = 0, 1
 class ConvDesc(C.Structure):
     _fields_ = [(n, C.c_int) for n in ('B', 'D', 'H', 'W', 'Cin', 'in_cstride', 'in_coff', 'Cout', 'kd', 'kh', 'kw',
                                        'stride', 'pd', 'ph', 'pw', 'Do', 'Ho', 'Wo', 'out_cstride', 'out_coff',
-                                       'prologue')] + [('group_rows', C.c_longlong), ('act', C.c_int), ('max_chain_k', C.c_int)]
+                                       'prologue')] + [('group_rows', C.c_longlong), ('act', C.c_int), ('max_chain_k', C.c_int),
+                                                           ('in_items', C.c_int)]
 
 
 class DetMaps(C.Structure):
@@ -92,14 +93,14 @@ _SIGNATURES = {
     'g6d_det_parse': [P, P, P, I, I, I, I, P, P, P],
     'g6d_det_corr_rowsum': [P, P, I, I, I, I, I, P],
     'g6d_sel_ref_sums': [P, I, I, I, P, P, P],
-    'g6d_sel_corr_prologue': [P, P, P, I, I, I, F, P, P, P],
+    'g6d_sel_corr_prologue': [P, P, P, I, I, I, I, F, P, P, P],
     'g6d_sel_corr_score': [P, P, I, I, I, P, P],
-    'g6d_sel_corr_score3': [P, P, P, P, P, P, I, I, I, I, I, P, P, P, P],
-    'g6d_sel_corr_score3_workspace_bytes': [I, I, I, I],
-    'g6d_sel_vp_norm': [P, I, I, F, P, I, I, P],
-    'g6d_sel_max_angle_add': [P, P, P, I, I, I, P],
-    'g6d_attention': [P, P, P, P, I, I, I, P],
-    'g6d_attention_headmajor': [P, P, P, P, I, I, I, P],
+    'g6d_sel_corr_score3': [P, P, P, P, P, P, I, I, I, I, I, I, P, P, P, P],
+    'g6d_sel_corr_score3_workspace_bytes': [I, I, I, I, I],
+    'g6d_sel_vp_norm': [P, I, I, I, F, P, I, I, P],
+    'g6d_sel_max_angle_add': [P, P, P, I, I, I, I, P],
+    'g6d_attention': [P, P, P, P, I, I, I, I, P],
+    'g6d_attention_headmajor': [P, P, P, P, I, I, I, I, P],
     'g6d_layernorm': [P, P, P, P, I, I, F, P],
     'g6d_sel_parse': [P, P, I, I, P, P, P],
     'g6d_ref_volume_fill': [P, P, P, P, P, P, I, I, I, I, I, I, I, I, P, P, P],

@@ -62,4 +62,15 @@ __device__ __forceinline__ float4 ldg_stream(const float4* p) {
 
 inline int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
 
+// g6d_conv_desc.in_items: 0 (one input item per output item) or a divisor of B (the input is broadcast)
+inline bool in_items_ok(const g6d_conv_desc* d) { return d->in_items == 0 || (d->in_items > 0 && d->B % d->in_items == 0); }
+// the conv kernels index the prologue operands (scale [groups, (D*H*W,) Cin]) with 32-bit offsets
+inline bool pro_operands_fit(const g6d_conv_desc* d) {
+    if (d->prologue == G6D_PRO_NONE) return true;
+    const long long gr = d->group_rows > 0 ? d->group_rows : 1;
+    const long long groups = (d->B + gr - 1) / gr;
+    const long long per = d->prologue == G6D_PRO_CORR ? (long long)d->D * d->H * d->W : 1;
+    return groups * per * d->Cin < (1ll << 31);
+}
+
 }  // namespace g6d

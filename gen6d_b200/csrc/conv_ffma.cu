@@ -18,6 +18,7 @@ struct ConvP {
     float* y; float* ws;
     int B, D, H, W, Cin, ics, ico, Cout, ldw, kd, kh, kw, stride, pd, ph, pw, Do, Ho, Wo, ocs, oco, pro, act;
     long long group_rows;
+    int in_items;             // input items: output item b reads input item b % in_items
     int M, K, ktiles, splits, kt_per_split;
 };
 
@@ -48,7 +49,8 @@ __global__ void __launch_bounds__(NT, 2) conv_ffma_kernel(const ConvP p) {
 
     // ---- A loader state: 2 rows per thread, one float4 (4 consecutive k) each
     const int kq = t & 3;
-    int rb[2], rz[2], ry[2], rx[2];
+    // rb: the input item a row reads; rg: the prologue group of its output item (once per tile, no divide in the K loop)
+    int rb[2], rg[2], rz[2], ry[2], rx[2];
     bool rvalid[2];
 #pragma unroll
     for (int i = 0; i < 2; ++i) {
@@ -58,7 +60,8 @@ __global__ void __launch_bounds__(NT, 2) conv_ffma_kernel(const ConvP p) {
         int xo = mm % p.Wo; mm /= p.Wo;
         int yo = mm % p.Ho; mm /= p.Ho;
         int zo = mm % p.Do; mm /= p.Do;
-        rb[i] = mm;
+        rb[i] = p.in_items == p.B ? mm : mm % p.in_items;
+        rg[i] = p.pro == G6D_PRO_NONE ? 0 : (int)(mm / p.group_rows);
         rz[i] = zo * p.stride - p.pd;
         ry[i] = yo * p.stride - p.ph;
         rx[i] = xo * p.stride - p.pw;
@@ -87,14 +90,13 @@ __global__ void __launch_bounds__(NT, 2) conv_ffma_kernel(const ConvP p) {
                 v = __ldg(reinterpret_cast<const float4*>(p.x + pos * p.ics + p.ico + c));
                 if (p.pro != G6D_PRO_NONE) {
                     float4 s, b;
+                    const int gc = rg[i] * p.Cin + c;                   // 32-bit (host checks the range)
                     if (p.pro == G6D_PRO_CORR) {
-                        const long long sp = ((long long)zi * p.H + yi) * p.W + xi;
-                        s = __ldg(reinterpret_cast<const float4*>(p.ps + sp * p.Cin + c));
-                        b = __ldg(reinterpret_cast<const float4*>(p.pb + c));
+                        s = __ldg(reinterpret_cast<const float4*>(p.ps + (((rg[i] * p.D + zi) * p.H + yi) * p.W + xi) * p.Cin + c));
+                        b = __ldg(reinterpret_cast<const float4*>(p.pb + gc));
                     } else {
-                        const long long g = rb[i] / p.group_rows;
-                        s = __ldg(reinterpret_cast<const float4*>(p.ps + g * p.Cin + c));
-                        b = __ldg(reinterpret_cast<const float4*>(p.pb + g * p.Cin + c));
+                        s = __ldg(reinterpret_cast<const float4*>(p.ps + gc));
+                        b = __ldg(reinterpret_cast<const float4*>(p.pb + gc));
                     }
                     v.x = fmaf(v.x, s.x, b.x); v.y = fmaf(v.y, s.y, b.y);
                     v.z = fmaf(v.z, s.z, b.z); v.w = fmaf(v.w, s.w, b.w);
@@ -347,6 +349,8 @@ static int fill_params(const g6d_conv_desc* d, ConvP& p) {
                 "g6d_conv: Cin (%d), in_cstride (%d), in_coff (%d) must be multiples of 4", d->Cin, d->in_cstride,
                 d->in_coff);
     G6D_REQUIRE(d->in_coff + d->Cin <= d->in_cstride, "g6d_conv: input channel slice out of row");
+    G6D_REQUIRE(in_items_ok(d), "g6d_conv: in_items (%d) must be 0 or divide B (%d)", d->in_items, d->B);
+    G6D_REQUIRE(pro_operands_fit(d), "g6d_conv: prologue operands too large");
     G6D_REQUIRE(d->out_coff + d->Cout <= d->out_cstride, "g6d_conv: output channel slice out of row");
     const int Do = (d->D + 2 * d->pd - d->kd) / d->stride + 1;
     const int Ho = (d->H + 2 * d->ph - d->kh) / d->stride + 1;
@@ -363,6 +367,7 @@ static int fill_params(const g6d_conv_desc* d, ConvP& p) {
     p.Cout = d->Cout; p.ldw = (d->Cout + 3) & ~3; p.kd = d->kd; p.kh = d->kh; p.kw = d->kw; p.stride = d->stride;
     p.pd = d->pd; p.ph = d->ph; p.pw = d->pw; p.Do = Do; p.Ho = Ho; p.Wo = Wo; p.ocs = d->out_cstride;
     p.oco = d->out_coff; p.pro = d->prologue; p.act = d->act; p.group_rows = d->group_rows > 0 ? d->group_rows : 1;
+    p.in_items = d->in_items > 0 ? d->in_items : d->B;
     p.M = (int)M; p.K = (int)K; p.ktiles = (int)((K + BK - 1) / BK);
     // split-K heuristic: fill ~2 CTAs per SM when the MN grid alone cannot
     const int bn = d->Cout > 64 ? 128 : (d->Cout > 32 ? 64 : 32);
@@ -400,7 +405,8 @@ extern "C" int g6d_conv(const g6d_conv_desc* desc, const float* x, const float* 
     p.x = x; p.w = w; p.bias = bias; p.ps = pro_scale; p.pb = pro_shift; p.y = y; p.ws = (float*)ws;
     cudaStream_t st = as_stream(stream);
     if (p.Cin == 4 && p.ics == 4 && p.ico == 0 && p.Cout == 64 && p.ocs == 64 && p.oco == 0 && p.kd == 1 && p.kh == 3 &&
-        p.kw == 3 && p.stride == 1 && p.pd == 0 && p.ph == 1 && p.pw == 1 && p.D == 1 && p.pro == G6D_PRO_NONE) {
+        p.kw == 3 && p.stride == 1 && p.pd == 0 && p.ph == 1 && p.pw == 1 && p.D == 1 && p.pro == G6D_PRO_NONE &&
+        p.in_items == p.B) {
         conv3x3_c4_o64_kernel<<<ceil_div(p.M, 128), 128, 0, st>>>(x, w, bias, y, p.B, p.H, p.W, p.act);
         G6D_CHECK_LAUNCH("g6d_conv(first layer)");
         return G6D_OK;

@@ -80,6 +80,7 @@ struct ConvTcP {
     float* y; float* ws;
     int B, D, H, W, Cin, ics, ico, Cout, kd, kh, kw, stride, pd, ph, pw, Do, Ho, Wo, ocs, oco, pro, act;
     long long group_rows;
+    int in_items;                             // input items: output item b reads input item b % in_items
     int M, K, kblocks, splits, kb_per_split;
     double* stats; long long stats_rows;      // fused InstanceNorm statistics of the OUTPUT (see epilogue_stats)
 };
@@ -299,8 +300,13 @@ conv_tc2_kernel(const ConvTcP p, const Tc2Work wk, const __grid_constant__ CUten
             const int m_base = mt * TC_BM;
             const int kb_begin = sp * p.kb_per_split;
             const int nkb = min(p.kblocks, kb_begin + p.kb_per_split) - kb_begin;
-            int rb[ROWS], rsp[ROWS], rc[ROWS];
-            unsigned rvmask = 0;
+            // Once per tile, so that the K-block loop has no divide: rin = the row's first tap as an input row index
+            // (input item * plane + spatial offset); byte j of gd = row j's prologue group minus g0 (bits 0-6; the
+            // rows are at most RSTEP * (ROWS - 1) < 128 apart) and its valid flag (bit 7).  The producers sit at the
+            // 128-register cap: this is fewer live registers than the (item, spatial offset) pair per row it replaces.
+            static_assert(ROWS <= 4 && RSTEP * (ROWS - 1) < 128, "group deltas must fit 7 bits each");
+            int rin[ROWS], rc[ROWS];
+            int g0 = 0; unsigned gd = 0;
             const long long plane_sz = (long long)p.D * p.H * p.W;
 #pragma unroll
             for (int j = 0; j < ROWS; ++j) {
@@ -310,11 +316,13 @@ conv_tc2_kernel(const ConvTcP p, const Tc2Work wk, const __grid_constant__ CUten
                 const int xo = m % p.Wo; m /= p.Wo;
                 const int yo = m % p.Ho; m /= p.Ho;
                 const int zo = m % p.Do; m /= p.Do;
-                rb[j] = m;
+                const int item = p.in_items == p.B ? m : m % p.in_items;
+                const int g = m / (int)p.group_rows;                                  // 32-bit divide (host checks the range)
+                if (j == 0) g0 = g;
+                if (v) gd |= ((unsigned)(g - g0) | 0x80u) << (8 * j);
                 const int z = zo * p.stride - p.pd, y = yo * p.stride - p.ph, x = xo * p.stride - p.pw;
-                rsp[j] = (z * p.H + y) * p.W + x;
+                rin[j] = item * (int)plane_sz + (z * p.H + y) * p.W + x;        // < 2^31 (host checks)
                 rc[j] = ((z + 8) << 24) | ((y + 8) << 12) | (x + 8);
-                if (v) rvmask |= 1u << j;
             }
             int c0, kx, ky, kz;
             {
@@ -333,12 +341,12 @@ conv_tc2_kernel(const ConvTcP p, const Tc2Work wk, const __grid_constant__ CUten
 #pragma unroll
                 for (int j = 0; j < ROWS; ++j) {
                     const int z = ((rc[j] >> 24) & 0xff) - 8 + kz, y = ((rc[j] >> 12) & 0xfff) - 8 + ky, x = (rc[j] & 0xfff) - 8 + kx;
-                    const bool inb = ((rvmask >> j) & 1u) && (unsigned)z < (unsigned)p.D && (unsigned)y < (unsigned)p.H &&
+                    const bool inb = ((gd >> (8 * j + 7)) & 1u) && (unsigned)z < (unsigned)p.D && (unsigned)y < (unsigned)p.H &&
                                      (unsigned)x < (unsigned)p.W;
 #pragma unroll
                     for (int e = 0; e < NV; ++e) v[q][j][e] = make_float4(0.f, 0.f, 0.f, 0.f);
                     if (inb) {
-                        const float4* src = reinterpret_cast<const float4*>(xb + ((long long)rb[j] * plane_sz + rsp[j] + tap_sp) * p.ics);
+                        const float4* src = reinterpret_cast<const float4*>(xb + (long long)(rin[j] + tap_sp) * p.ics);
 #pragma unroll
                         for (int e = 0; e < NV; ++e) v[q][j][e] = __ldg(src + e * 8);
                         okm[q] |= 1u << j;
@@ -357,14 +365,15 @@ conv_tc2_kernel(const ConvTcP p, const Tc2Work wk, const __grid_constant__ CUten
                     for (int j = 0; j < ROWS; ++j) {
                         if (okm[q] & (1u << j)) {
                             const float4* scp; const float4* shp;
-                            if (p.pro == G6D_PRO_CORR) {
-                                scp = reinterpret_cast<const float4*>(p.ps + (long long)(rsp[j] + ksp[q]) * p.Cin + kc[q]);
-                                shp = reinterpret_cast<const float4*>(p.pb + kc[q]);
+                            const int gc = (g0 + (int)((gd >> (8 * j)) & 0x7fu)) * p.Cin;
+                            const int sh = gc + kc[q];
+                            if (p.pro == G6D_PRO_CORR) {       // scale[g, pos, c]: the spatial offset again from rc
+                                const int rsp = ((((rc[j] >> 24) & 0xff) - 8) * p.H + ((rc[j] >> 12) & 0xfff) - 8) * p.W + (rc[j] & 0xfff) - 8;
+                                scp = reinterpret_cast<const float4*>(p.ps + (gc * (int)plane_sz + (rsp + ksp[q]) * p.Cin + kc[q]));
                             } else {
-                                const long long g = rb[j] / (int)p.group_rows;       // 32-bit divide (host checks the range)
-                                scp = reinterpret_cast<const float4*>(p.ps + g * p.Cin + kc[q]);
-                                shp = reinterpret_cast<const float4*>(p.pb + g * p.Cin + kc[q]);
+                                scp = reinterpret_cast<const float4*>(p.ps + sh);
                             }
+                            shp = reinterpret_cast<const float4*>(p.pb + sh);
 #pragma unroll
                             for (int e = 0; e < NV; ++e) v[q][j][e] = affine4(v[q][j][e], __ldg(scp + e * 8), __ldg(shp + e * 8), relu);
                         }
@@ -667,7 +676,8 @@ static int tc_block_n(int Cout) { return Cout > 64 ? 128 : (Cout > 32 ? 64 : 32)
 // the persistent kernel packs (z, y, x) + 8 into 8/12/12 bits and uses 32-bit spatial offsets and group indices
 static bool tc2_dims_ok(const g6d_conv_desc* d) {
     return d->D + d->pd + 8 < 256 && d->H + d->ph + 8 < 4096 && d->W + d->pw + 8 < 4096 &&
-           (long long)d->D * d->H * d->W < (1ll << 30) && d->group_rows < (1ll << 31);
+           (long long)d->D * d->H * d->W < (1ll << 30) && d->group_rows < (1ll << 31) &&
+           (long long)(d->in_items > 0 ? d->in_items : d->B) * d->D * d->H * d->W < (1ll << 31);
 }
 
 static int fill_tc_params(const g6d_conv_desc* d, int kind, ConvTcP& p) {
@@ -680,6 +690,8 @@ static int fill_tc_params(const g6d_conv_desc* d, int kind, ConvTcP& p) {
     G6D_REQUIRE((d->in_cstride & 3) == 0 && (d->in_coff & 3) == 0, "g6d_conv_tc: in_cstride/in_coff must be multiples of 4");
     G6D_REQUIRE(d->in_coff + d->Cin <= d->in_cstride, "g6d_conv_tc: input channel slice out of row");
     G6D_REQUIRE(d->out_coff + d->Cout <= d->out_cstride, "g6d_conv_tc: output channel slice out of row");
+    G6D_REQUIRE(in_items_ok(d), "g6d_conv_tc: in_items (%d) must be 0 or divide B (%d)", d->in_items, d->B);
+    G6D_REQUIRE(pro_operands_fit(d), "g6d_conv_tc: prologue operands too large");
     G6D_REQUIRE(tc2_dims_ok(d), "g6d_conv_tc: spatial extent too large for the tensor-core kernel");
     const int Do = (d->D + 2 * d->pd - d->kd) / d->stride + 1;
     const int Ho = (d->H + 2 * d->ph - d->kh) / d->stride + 1;
@@ -693,6 +705,7 @@ static int fill_tc_params(const g6d_conv_desc* d, int kind, ConvTcP& p) {
     p.Cout = d->Cout; p.kd = d->kd; p.kh = d->kh; p.kw = d->kw; p.stride = d->stride; p.pd = d->pd; p.ph = d->ph;
     p.pw = d->pw; p.Do = Do; p.Ho = Ho; p.Wo = Wo; p.ocs = d->out_cstride; p.oco = d->out_coff; p.pro = d->prologue;
     p.act = d->act; p.group_rows = d->group_rows > 0 ? d->group_rows : 1;
+    p.in_items = d->in_items > 0 ? d->in_items : d->B;
     p.M = (int)M; p.K = (int)K; p.kblocks = (int)(K / bk);
     const int bn = tc_block_n(d->Cout);
     const long long ctas = (long long)ceil_div(M, TC_BM) * ceil_div(d->Cout, bn);
@@ -807,6 +820,7 @@ struct ConvFlatP {
     const float* x; const float* bias; const float* ps; const float* pb; float* y; float* ws;
     int B, D, H, W, Cin, ics, ico, Cout, kd, kh, kw, pd, ph, pw, Do, Ho, Wo, ocs, oco, pro, act;
     long long group_rows;
+    int in_items;
     int Wp, tiles_per_plane, mode, nseg, taps_per_seg, seg_rows, rows_pad, ntab, cblocks;
     int a_stages, b_stages, splits, cb_per_split, M;
     double* stats; long long stats_rows;
@@ -892,7 +906,8 @@ conv_tcflat_kernel(const ConvFlatP p, const __grid_constant__ CUtensorMap map_hi
         const int cofs = chunk * 4;                             // channels [cofs, cofs+4) (+32 for the 2nd load), see f16_k_source
         const int r0 = threadIdx.x >> 3;                        // rows r0 + 32*j
         const long long plane = (long long)p.H * p.W;
-        const long long gi = (long long)b / p.group_rows;
+        const long long gi = (long long)b / p.group_rows;        // prologue group of the output item
+        const int b_in = p.in_items == p.B ? b : b % p.in_items;  // the input item it reads
         const bool relu = p.pro == G6D_PRO_AFFINE_RELU;
         // Software pipeline over (unit, 128-row trip) with a ring of NB register slots: the global loads of
         // the next NB-1 trips (possibly of the next unit: they only touch registers, so they do not wait for
@@ -915,7 +930,7 @@ conv_tcflat_kernel(const ConvFlatP p, const __grid_constant__ CUtensorMap map_hi
             unit_of(tt, u, rbase, cb, kz, tb);
             const int zz = zo + kz - p.pd;
             const bool zok = (unsigned)zz < (unsigned)p.D;
-            const float* xplane = p.x + ((long long)b * p.D + (zok ? zz : 0)) * plane * p.ics + p.ico + cb * BK + cofs;
+            const float* xplane = p.x + ((long long)b_in * p.D + (zok ? zz : 0)) * plane * p.ics + p.ico + cb * BK + cofs;
             const int* tab = rowtab + tb * p.seg_rows;
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
@@ -944,9 +959,9 @@ conv_tcflat_kernel(const ConvFlatP p, const __grid_constant__ CUtensorMap map_hi
                 if (p.pro != G6D_PRO_NONE && off[q][j] >= 0) {
                     const float4* scp; const float4* shp;
                     if (p.pro == G6D_PRO_CORR) {
-                        const long long sp = (long long)zz * plane + off[q][j];
+                        const long long sp = (gi * p.D + zz) * plane + off[q][j];
                         scp = reinterpret_cast<const float4*>(p.ps + sp * p.Cin + c);
-                        shp = reinterpret_cast<const float4*>(p.pb + c);
+                        shp = reinterpret_cast<const float4*>(p.pb + gi * p.Cin + c);
                     } else {
                         scp = reinterpret_cast<const float4*>(p.ps + gi * p.Cin + c);
                         shp = reinterpret_cast<const float4*>(p.pb + gi * p.Cin + c);
@@ -1120,7 +1135,7 @@ static bool flat_disabled() { return flat_level() == 0; }
 
 static int fill_flat_params(const g6d_conv_desc* d, int kind, ConvFlatP& p, int* smem_bytes) {
     const int bk = kind_bk(kind);
-    if (!d || d->stride != 1 || (d->Cin % bk) != 0 || d->Cout < 16 || (d->in_cstride & 3) || (d->in_coff & 3)) return -1;
+    if (!d || !in_items_ok(d) || d->stride != 1 || (d->Cin % bk) != 0 || d->Cout < 16 || (d->in_cstride & 3) || (d->in_coff & 3)) return -1;
     const int Do = d->D + 2 * d->pd - d->kd + 1, Ho = d->H + 2 * d->ph - d->kh + 1, Wo = d->W + 2 * d->pw - d->kw + 1;
     if (Do != d->Do || Ho != d->Ho || Wo != d->Wo || Do < 1 || Ho < 1 || Wo < 1) return -1;
     if (d->kd * d->kh * d->kw == 1) return -1;                        // 1x1: nothing to reuse, persistent kernel
@@ -1146,6 +1161,7 @@ static int fill_flat_params(const g6d_conv_desc* d, int kind, ConvFlatP& p, int*
     p.Cout = d->Cout; p.kd = d->kd; p.kh = d->kh; p.kw = d->kw; p.pd = d->pd; p.ph = d->ph; p.pw = d->pw;
     p.Do = Do; p.Ho = Ho; p.Wo = Wo; p.ocs = d->out_cstride; p.oco = d->out_coff; p.pro = d->prologue; p.act = d->act;
     p.group_rows = d->group_rows > 0 ? d->group_rows : 1;
+    p.in_items = d->in_items > 0 ? d->in_items : d->B;
     p.Wp = Wp; p.tiles_per_plane = (Ho * Wp + TC_BM - 1) / TC_BM; p.mode = mode;
     p.nseg = mode == 0 ? d->kd : d->kd * d->kh; p.taps_per_seg = mode == 0 ? d->kh * d->kw : d->kw;
     p.seg_rows = rows; p.rows_pad = (rows + 7) / 8 * 8; p.ntab = ntab; p.cblocks = d->Cin / bk;
@@ -1222,7 +1238,7 @@ extern "C" int g6d_conv_tc_debug(int* host_out8) {
 
 extern "C" int g6d_conv_tc_supported(const g6d_conv_desc* d, int kind) {
     if (!d || (kind != G6D_TC_TF32 && kind != G6D_TC_F16)) return 0;
-    return (d->Cin % kind_bk(kind)) == 0 && d->Cout >= 16 && (d->in_cstride & 3) == 0 && (d->in_coff & 3) == 0 &&
+    return in_items_ok(d) && pro_operands_fit(d) && (d->Cin % kind_bk(kind)) == 0 && d->Cout >= 16 && (d->in_cstride & 3) == 0 && (d->in_coff & 3) == 0 &&
            tc2_dims_ok(d) ? 1 : 0;
 }
 

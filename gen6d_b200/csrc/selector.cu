@@ -64,28 +64,32 @@ __global__ void __launch_bounds__(256) sel_corr_score_kernel(const float* __rest
 }
 
 // ------------------------------------------------------------------------------------------
-// S2, all pyramid levels in ONE streaming pass (what select_que_imgs uses): phase 1 computes
-// every per-location inner product t[row] for row = (level, slice, location) with a grid-stride
-// loop over rows -- the grid is sized to fill every SM with 64 resident warps regardless of S, and
-// each warp keeps two 2 KB rows (8 x 128-bit loads per lane) in flight; phase 2 (tiny, L2-resident)
-// reduces each (level, slice) to sum_p t*(t/max_p t).
+// S2, all pyramid levels and all qn queries in ONE streaming pass (what select_que_imgs uses):
+// phase 1 computes every per-location inner product t[g, row] for row = (level, slice, location)
+// with a grid-stride loop over rows -- the grid is sized to fill every SM with 32 resident warps
+// regardless of S (64 registers: the two rows stay in registers across the query loop), and each
+// warp keeps two 2 KB reference rows (8 x 128-bit loads per lane, 128 KB per SM) in flight and
+// dots them with the rows of all qn queries (small, L2-resident), so the reference
+// stack is read from HBM once per batch, not once per query; phase 2 (tiny, L2-resident) reduces
+// each (query, level, slice) to sum_p t*(t/max_p t).
 struct ScoreLevels {
     const float* ref[3];   // [S, P_l, C]
-    const float* q[3];     // [P_l, C]
+    const float* q[3];     // [qn, P_l, C]
     int P[3];
-    int S;
+    int S, qn;
     long long row_end[3];  // cumulative row counts: S*P_0, S*(P_0+P_1), S*(P_0+P_1+P_2)
 };
 
 template <int C>
-__device__ __forceinline__ float row_dot(const float4* __restrict__ rp, const float4* __restrict__ qp, int lane) {
-    constexpr int V = C / 128;
-    float4 rv[V];
+__device__ __forceinline__ void row_load(const float4* __restrict__ rp, int lane, float4 (&rv)[C / 128]) {
 #pragma unroll
-    for (int i = 0; i < V; ++i) rv[i] = ldg_stream(rp + lane + 32 * i);
+    for (int i = 0; i < C / 128; ++i) rv[i] = ldg_stream(rp + lane + 32 * i);
+}
+template <int C>
+__device__ __forceinline__ float row_dot(const float4 (&rv)[C / 128], const float4* __restrict__ qp, int lane) {
     float t = 0.f;
 #pragma unroll
-    for (int i = 0; i < V; ++i) {
+    for (int i = 0; i < C / 128; ++i) {
         const float4 qv = __ldg(qp + lane + 32 * i);
         t = fmaf(rv[i].x, qv.x, fmaf(rv[i].y, qv.y, fmaf(rv[i].z, qv.z, fmaf(rv[i].w, qv.w, t))));
     }
@@ -93,12 +97,13 @@ __device__ __forceinline__ float row_dot(const float4* __restrict__ rp, const fl
 }
 
 // FUSED: every CTA streams one CONTIGUOUS chunk of rows, then (one __threadfence per warp, one
-// __syncthreads) adds the rows it contributed to each (level, slice) item it touched to that item's
-// completion counter; the CTA that completes an item reduces its P inner products to the score with
-// the reference's operation order (selector.py:192-194: s / max first, then sum of s * (s / max); IEEE
-// behaviour for max <= 0, no epsilon).  ~6 atomics per CTA, no second launch.
+// __syncthreads) adds the rows it contributed to each (query, level, slice) item it touched to that
+// item's completion counter; the CTA that completes an item reduces its P inner products to the score
+// with the reference's operation order (selector.py:192-194: s / max first, then sum of s * (s / max);
+// IEEE behaviour for max <= 0, no epsilon).  ~6 qn atomics per CTA, no second launch.  t_out is
+// [qn, rows], score [qn, 3, S], done [qn, 3, S].
 template <int C, bool FUSED>
-__global__ void __launch_bounds__(256, 6) sel_corr_dots_kernel(const ScoreLevels L, float* __restrict__ t_out,
+__global__ void __launch_bounds__(256, 4) sel_corr_dots_kernel(const ScoreLevels L, float* __restrict__ t_out,
                                                             int* __restrict__ done, float* __restrict__ score,
                                                             long long chunk) {
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -116,7 +121,7 @@ __global__ void __launch_bounds__(256, 6) sel_corr_dots_kernel(const ScoreLevels
         item = (l0 ? 0 : (l1 ? 1 : 2)) * L.S + sl;
         first = lbase + (long long)sl * P;
         rp = reinterpret_cast<const float4*>(ref + local * C);
-        qp = reinterpret_cast<const float4*>(q + (long long)p * C);
+        qp = reinterpret_cast<const float4*>(q + (long long)p * C);              // query 0; query g at + g*P*C
     };
     long long begin, end, stride;
     if (FUSED) {        // contiguous chunk per CTA, row pairs dealt to its 8 warps
@@ -134,63 +139,73 @@ __global__ void __launch_bounds__(256, 6) sel_corr_dots_kernel(const ScoreLevels
         long long first;
         locate(row, r0, q0, item, P, first);
         const bool two = row + 1 < end;
+        const int P0 = P;
         locate(two ? row + 1 : row, r1, q1, item, P, first);
-        float t0 = row_dot<C>(r0, q0, lane);
-        float t1 = row_dot<C>(r1, q1, lane);
-        t0 = warp_sum(t0);
-        t1 = warp_sum(t1);
-        if (lane == 0) {
-            t_out[row] = t0;
-            if (two) t_out[row + 1] = t1;
+        float4 v0[C / 128], v1[C / 128];
+        row_load<C>(r0, lane, v0);
+        row_load<C>(r1, lane, v1);
+        // same products and summation order for every query as a one-query call: bit-identical t
+        for (int g = 0; g < L.qn; ++g) {
+            float t0 = row_dot<C>(v0, q0 + (long long)g * P0 * (C / 4), lane);
+            float t1 = row_dot<C>(v1, q1 + (long long)g * P * (C / 4), lane);
+            t0 = warp_sum(t0);
+            t1 = warp_sum(t1);
+            if (lane == 0) {
+                t_out[g * rows + row] = t0;
+                if (two) t_out[g * rows + row + 1] = t1;
+            }
         }
     }
     if (!FUSED) return;
     if (lane == 0) __threadfence();                // this warp's t values are visible device-wide ...
     __syncthreads();                               // ... before any thread of the CTA counts them in
-    // the items this chunk overlaps, dealt round-robin to the warps
+    // the (item, query) pairs this chunk overlaps, dealt round-robin to the warps
     int n = 0;
-    for (long long r = begin; r < end; ++n) {
+    for (long long r = begin; r < end;) {
         const float4 *rp, *qp;
         int item, P;
         long long first;
         locate(r, rp, qp, item, P, first);
         const long long next = min(end, first + P);
-        if ((n & 7) == wib) {
+        for (int g = 0; g < L.qn; ++g, ++n) {
+            if ((n & 7) != wib) continue;
+            const long long gi = (long long)g * 3 * L.S + item;
             int last = 0;
-            if (lane == 0) last = atomicAdd(done + item, (int)(next - r)) + (int)(next - r) == P;
+            if (lane == 0) last = atomicAdd(done + gi, (int)(next - r)) + (int)(next - r) == P;
             last = __shfl_sync(0xffffffffu, last, 0);
             if (last) {                                                   // warp-uniform
-                if (lane == 0) done[item] = 0;                            // leave the counters zero for the next call
+                if (lane == 0) done[gi] = 0;                              // leave the counters zero for the next call
                 __threadfence();                                          // acquire: the other CTAs' t values
-                const float* tp = t_out + first;
+                const float* tp = t_out + g * rows + first;
                 float m = -INFINITY;
                 for (int p = lane; p < P; p += 32) m = fmaxf(m, __ldcg(tp + p));
                 m = warp_max(m);
                 float acc = 0.f;
                 for (int p = lane; p < P; p += 32) { const float v = __ldcg(tp + p); acc += v * (v / m); }
                 acc = warp_sum(acc);
-                if (lane == 0) score[item] = acc;       // [3, S]
+                if (lane == 0) score[gi] = acc;         // [qn, 3, S]
             }
         }
         r = next;
     }
 }
 
-// one warp per (level, slice): score = sum_p t*(t/max_p t), reference operation order (unfused path)
+// one warp per (query, level, slice): score = sum_p t*(t/max_p t), reference operation order (unfused path)
 __global__ void sel_corr_finish_kernel(const ScoreLevels L, const float* __restrict__ t, float* __restrict__ score) {
     const int lane = threadIdx.x & 31;
     const int item = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-    if (item >= 3 * L.S) return;
-    const int l = item / L.S, s = item % L.S;
+    if (item >= 3 * L.S * L.qn) return;
+    const int g = item / (3 * L.S), li = item % (3 * L.S);
+    const int l = li / L.S, s = li % L.S;
     const int P = l == 0 ? L.P[0] : (l == 1 ? L.P[1] : L.P[2]);
-    const float* tp = t + (l == 0 ? 0 : (l == 1 ? L.row_end[0] : L.row_end[1])) + (long long)s * P;
+    const float* tp = t + g * L.row_end[2] + (l == 0 ? 0 : (l == 1 ? L.row_end[0] : L.row_end[1])) + (long long)s * P;
     float m = -INFINITY;
     for (int p = lane; p < P; p += 32) m = fmaxf(m, tp[p]);
     m = warp_max(m);
     float acc = 0.f;
     for (int p = lane; p < P; p += 32) { const float v = tp[p]; acc += v * (v / m); }
     acc = warp_sum(acc);
-    if (lane == 0) score[item] = acc;       // [3, S]
+    if (lane == 0) score[item] = acc;       // [qn, 3, S]
 }
 
 // ------------------------------------------------------------------------------------------
@@ -209,11 +224,14 @@ __global__ void sel_ref_sums_kernel(const float* __restrict__ ref, int S, long l
     atomicAdd(sum2 + i, b);
 }
 
-// Per channel c: mean_c = sum_p q[p,c]*A[p,c] / N, E2_c = sum_p q[p,c]^2*B[p,c] / N, N = S*P;
-// then scale[p,c] = q[p,c]*rstd_c and shift[c] = -mean_c*rstd_c.  One block per 32 channels.
+// Per query g and channel c: mean_c = sum_p q[p,c]*A[p,c] / N, E2_c = sum_p q[p,c]^2*B[p,c] / N, N = S*P;
+// then scale[p,c] = q[p,c]*rstd_c and shift[c] = -mean_c*rstd_c.  One block per (32 channels, query).
 __global__ void sel_corr_prologue_kernel(const float* __restrict__ q, const double* __restrict__ sum1,
                                          const double* __restrict__ sum2, int S, int P, int C, float eps,
                                          float* __restrict__ scale, float* __restrict__ shift) {
+    q += (long long)blockIdx.y * P * C;
+    scale += (long long)blockIdx.y * P * C;
+    shift += (long long)blockIdx.y * C;
     const int c = blockIdx.x * 32 + (threadIdx.x & 31);
     const int row = threadIdx.x >> 5, nrow = blockDim.x >> 5;
     __shared__ double sm[8][32], sv[8][32];
@@ -245,11 +263,12 @@ __global__ void sel_corr_prologue_kernel(const float* __restrict__ q, const doub
     }
 }
 
-// vp_norm: InstanceNorm2d over n values per level; scatter to feats[i, coff + l]
+// vp_norm: InstanceNorm2d over n values per (group, level); scatter to feats[g*n + i, coff + l].  Block (l, g).
 __global__ void sel_vp_norm_kernel(const float* __restrict__ score, int n, float eps, float* __restrict__ feats,
                                    int cstride, int coff) {
     const int l = blockIdx.x;
-    const float* s = score + (long long)l * n;
+    const float* s = score + ((long long)blockIdx.y * gridDim.x + l) * n;
+    feats += (long long)blockIdx.y * n * cstride;
     __shared__ double r1[32], r2[32];
     double a = 0.0, b = 0.0;
     for (int i = threadIdx.x; i < n; i += blockDim.x) { const double v = s[i]; a += v; b += v * v; }
@@ -265,21 +284,22 @@ __global__ void sel_vp_norm_kernel(const float* __restrict__ score, int n, float
     const float fm = (float)mean;
     for (int i = threadIdx.x; i < n; i += blockDim.x) feats[(long long)i * cstride + coff + l] = (s[i] - fm) * rstd;
     // the channels between the last score and the row end are padding the consumer multiplies by zero
-    // weights: they must be finite, so the first block clears them (no separate fill pass over feats)
+    // weights: they must be finite, so the first block of each group clears them (no separate fill pass over feats)
     if (l == 0)
         for (int c = coff + (int)gridDim.x; c < cstride; ++c)
             for (int i = threadIdx.x; i < n; i += blockDim.x) feats[(long long)i * cstride + c] = 0.f;
 }
 
+// rows = groups * rfn; the embedding [rfn, C] is shared by every group
 __global__ void sel_max_angle_add_kernel(const float* __restrict__ x, const float* __restrict__ embed,
-                                         float* __restrict__ out, int rfn, int an, int C) {
+                                         float* __restrict__ out, int rows, int rfn, int an, int C) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (long long)rfn * C) return;
+    if (i >= (long long)rows * C) return;
     const int c = (int)(i % C);
     const int r = (int)(i / C);
     float m = -INFINITY;
     for (int a = 0; a < an; ++a) m = fmaxf(m, x[((long long)r * an + a) * C + c]);
-    out[i] = m + embed[i];
+    out[i] = m + embed[(long long)(r % rfn) * C + c];
 }
 
 // attention: one block per (query token i, head h); channel c = d*heads + h.
@@ -288,6 +308,8 @@ __global__ void attention_kernel(const float* __restrict__ q, const float* __res
                                  float* __restrict__ out, int n, int C, int heads) {
     extern __shared__ float sh[];  // [n] probabilities + [D] query
     const int i = blockIdx.x, h = blockIdx.y;
+    const long long go = (long long)blockIdx.z * n * C;      // group: n tokens of its own
+    q += go; k += go; v += go; out += go;
     const int D = C / heads;
     float* prob = sh;
     float* qv = sh + n;
@@ -341,6 +363,8 @@ __global__ void __launch_bounds__(128) attention_hm_kernel(const float* __restri
     __shared__ float s_sum[ATT_TQ];
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
     const int i0 = blockIdx.x * ATT_TQ, h = blockIdx.y;
+    const long long go = (long long)blockIdx.z * n * C;      // group: n tokens of its own
+    q += go; k += go; v += go; out += go;
     const float inv = rsqrtf((float)ATT_D);
     for (int e = t; e < ATT_TQ * ATT_D; e += 128) {
         const int qi = e / ATT_D, d = e % ATT_D;
@@ -457,21 +481,22 @@ extern "C" int g6d_sel_corr_score(const float* ref, const float* q, int S, int P
     return G6D_OK;
 }
 
-extern "C" long long g6d_sel_corr_score3_workspace_bytes(int S, int P0, int P1, int P2) {
-    if (S <= 0 || P0 <= 0 || P1 <= 0 || P2 <= 0) { set_error("g6d_sel_corr_score3_workspace_bytes: bad args"); return -1; }
-    const long long rows = (long long)S * ((long long)P0 + P1 + P2);
+extern "C" long long g6d_sel_corr_score3_workspace_bytes(int S, int P0, int P1, int P2, int qn) {
+    if (S <= 0 || P0 <= 0 || P1 <= 0 || P2 <= 0 || qn <= 0) { set_error("g6d_sel_corr_score3_workspace_bytes: bad args"); return -1; }
+    const long long rows = (long long)qn * S * ((long long)P0 + P1 + P2);
     return ((rows + 3) / 4) * 4 * (long long)sizeof(float);
 }
 
 extern "C" int g6d_sel_corr_score3(const float* ref0, const float* ref1, const float* ref2, const float* q0,
-                                   const float* q1, const float* q2, int S, int P0, int P1, int P2, int C, float* score,
-                                   float* ws, int* counters, g6d_stream_t stream) {
-    G6D_REQUIRE(ref0 && ref1 && ref2 && q0 && q1 && q2 && score && ws && S > 0 && P0 > 0 && P1 > 0 && P2 > 0,
+                                   const float* q1, const float* q2, int S, int P0, int P1, int P2, int C, int qn,
+                                   float* score, float* ws, int* counters, g6d_stream_t stream) {
+    G6D_REQUIRE(ref0 && ref1 && ref2 && q0 && q1 && q2 && score && ws && S > 0 && P0 > 0 && P1 > 0 && P2 > 0 && qn > 0,
                 "g6d_sel_corr_score3: bad args");
     G6D_REQUIRE(C == 512, "g6d_sel_corr_score3: C must be 512 (got %d)", C);
+    G6D_REQUIRE(3ll * S * qn < (1ll << 31), "g6d_sel_corr_score3: too many (query, level, slice) items");
     ScoreLevels L;
     L.ref[0] = ref0; L.ref[1] = ref1; L.ref[2] = ref2; L.q[0] = q0; L.q[1] = q1; L.q[2] = q2;
-    L.P[0] = P0; L.P[1] = P1; L.P[2] = P2; L.S = S;
+    L.P[0] = P0; L.P[1] = P1; L.P[2] = P2; L.S = S; L.qn = qn;
     L.row_end[0] = (long long)S * P0; L.row_end[1] = L.row_end[0] + (long long)S * P1;
     L.row_end[2] = L.row_end[1] + (long long)S * P2;
     cudaStream_t st = as_stream(stream);
@@ -500,7 +525,7 @@ extern "C" int g6d_sel_corr_score3(const float* ref0, const float* ref1, const f
     }
     sel_corr_dots_kernel<512, false><<<(unsigned)grid, 256, 0, st>>>(L, ws, nullptr, nullptr, 0);
     G6D_CHECK_LAUNCH("g6d_sel_corr_score3(dots)");
-    sel_corr_finish_kernel<<<ceil_div(3ll * S * 32, 256), 256, 0, st>>>(L, ws, score);
+    sel_corr_finish_kernel<<<ceil_div(3ll * S * qn * 32, 256), 256, 0, st>>>(L, ws, score);
     G6D_CHECK_LAUNCH("g6d_sel_corr_score3(finish)");
     return G6D_OK;
 }
@@ -520,43 +545,48 @@ extern "C" int g6d_sel_ref_sums(const float* ref, int S, int P, int C, double* s
     return G6D_OK;
 }
 
-extern "C" int g6d_sel_corr_prologue(const float* q, const double* sum1, const double* sum2, int S, int P, int C,
+extern "C" int g6d_sel_corr_prologue(const float* q, const double* sum1, const double* sum2, int S, int P, int C, int qn,
                                      float eps, float* scale, float* shift, g6d_stream_t stream) {
-    G6D_REQUIRE(q && sum1 && sum2 && scale && shift && S > 0 && P > 0 && C > 0, "g6d_sel_corr_prologue: bad args");
-    sel_corr_prologue_kernel<<<ceil_div(C, 32), 256, 0, as_stream(stream)>>>(q, sum1, sum2, S, P, C, eps, scale, shift);
+    G6D_REQUIRE(q && sum1 && sum2 && scale && shift && S > 0 && P > 0 && C > 0 && qn > 0 && qn <= 65535,
+                "g6d_sel_corr_prologue: bad args");
+    sel_corr_prologue_kernel<<<dim3(ceil_div(C, 32), qn), 256, 0, as_stream(stream)>>>(q, sum1, sum2, S, P, C, eps, scale, shift);
     G6D_CHECK_LAUNCH("g6d_sel_corr_prologue");
     return G6D_OK;
 }
 
-extern "C" int g6d_sel_vp_norm(const float* score, int L, int n, float eps, float* feats, int cstride, int coff,
+extern "C" int g6d_sel_vp_norm(const float* score, int groups, int L, int n, float eps, float* feats, int cstride, int coff,
                                g6d_stream_t stream) {
-    G6D_REQUIRE(score && feats && L > 0 && n > 0 && coff + L <= cstride, "g6d_sel_vp_norm: bad args");
-    sel_vp_norm_kernel<<<L, 256, 0, as_stream(stream)>>>(score, n, eps, feats, cstride, coff);
+    G6D_REQUIRE(score && feats && groups > 0 && groups <= 65535 && L > 0 && n > 0 && coff + L <= cstride,
+                "g6d_sel_vp_norm: bad args");
+    sel_vp_norm_kernel<<<dim3(L, groups), 256, 0, as_stream(stream)>>>(score, n, eps, feats, cstride, coff);
     G6D_CHECK_LAUNCH("g6d_sel_vp_norm");
     return G6D_OK;
 }
 
-extern "C" int g6d_sel_max_angle_add(const float* x, const float* embed, float* out, int rfn, int an, int C,
+extern "C" int g6d_sel_max_angle_add(const float* x, const float* embed, float* out, int groups, int rfn, int an, int C,
                                      g6d_stream_t stream) {
-    G6D_REQUIRE(x && embed && out && rfn > 0 && an > 0 && C > 0, "g6d_sel_max_angle_add: bad args");
-    sel_max_angle_add_kernel<<<ceil_div((long long)rfn * C, 256), 256, 0, as_stream(stream)>>>(x, embed, out, rfn, an, C);
+    G6D_REQUIRE(x && embed && out && groups > 0 && rfn > 0 && an > 0 && C > 0 && (long long)groups * rfn < (1ll << 31),
+                "g6d_sel_max_angle_add: bad args");
+    const int rows = groups * rfn;
+    sel_max_angle_add_kernel<<<ceil_div((long long)rows * C, 256), 256, 0, as_stream(stream)>>>(x, embed, out, rows, rfn, an, C);
     G6D_CHECK_LAUNCH("g6d_sel_max_angle_add");
     return G6D_OK;
 }
 
-extern "C" int g6d_attention(const float* q, const float* k, const float* v, float* out, int n, int C, int heads,
+extern "C" int g6d_attention(const float* q, const float* k, const float* v, float* out, int groups, int n, int C, int heads,
                              g6d_stream_t stream) {
-    G6D_REQUIRE(q && k && v && out && n > 0 && n <= 8192 && heads > 0 && C % heads == 0, "g6d_attention: bad args");
+    G6D_REQUIRE(q && k && v && out && groups > 0 && groups <= 65535 && n > 0 && n <= 8192 && heads > 0 && C % heads == 0,
+                "g6d_attention: bad args");
     const size_t smem = sizeof(float) * (n + C / heads);
-    attention_kernel<<<dim3(n, heads), 64, smem, as_stream(stream)>>>(q, k, v, out, n, C, heads);
+    attention_kernel<<<dim3(n, heads, groups), 64, smem, as_stream(stream)>>>(q, k, v, out, n, C, heads);
     G6D_CHECK_LAUNCH("g6d_attention");
     return G6D_OK;
 }
 
-extern "C" int g6d_attention_headmajor(const float* q, const float* k, const float* v, float* out, int n, int C, int heads,
-                                       g6d_stream_t stream) {
-    G6D_REQUIRE(q && k && v && out && n > 0 && n <= 2048 && heads > 0 && C == heads * ATT_D && (C & 3) == 0,
-                "g6d_attention_headmajor: bad args (n <= 2048, C = heads * 64)");
+extern "C" int g6d_attention_headmajor(const float* q, const float* k, const float* v, float* out, int groups, int n, int C,
+                                       int heads, g6d_stream_t stream) {
+    G6D_REQUIRE(q && k && v && out && groups > 0 && groups <= 65535 && n > 0 && n <= 2048 && heads > 0 &&
+                C == heads * ATT_D && (C & 3) == 0, "g6d_attention_headmajor: bad args (n <= 2048, C = heads * 64)");
     const int npad = (n + 31) & ~31;
     const size_t smem = sizeof(float) * (ATT_TQ * ATT_D + ATT_TK * (ATT_D + 1) + (size_t)ATT_TQ * npad);
     static bool configured = false;
@@ -565,7 +595,7 @@ extern "C" int g6d_attention_headmajor(const float* q, const float* k, const flo
         if (e != cudaSuccess) { set_error("g6d_attention_headmajor: %s", cudaGetErrorString(e)); return G6D_ECUDA; }
         configured = true;
     }
-    attention_hm_kernel<<<dim3(ceil_div(n, ATT_TQ), heads), 128, smem, as_stream(stream)>>>(q, k, v, out, n, C);
+    attention_hm_kernel<<<dim3(ceil_div(n, ATT_TQ), heads, groups), 128, smem, as_stream(stream)>>>(q, k, v, out, n, C);
     G6D_CHECK_LAUNCH("g6d_attention_headmajor");
     return G6D_OK;
 }

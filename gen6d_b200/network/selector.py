@@ -142,17 +142,19 @@ class ViewpointSelector(PackedModule):
         self.bump_generation()          # captured graphs / worker clones hold pointers to the previous reference set
 
     def comm_stats(self):
-        """Collectives issued per query by the sharded path (counted on the last eager / capture pass)."""
+        """Collectives issued per select pass (one batch of queries) by the sharded path (counted on the last eager /
+        capture pass)."""
         return dict(getattr(self.comm, 'calls', {}))
 
-    def _s2_counters(self):
-        """Completion counters of the fused S2 kernel: zero between calls (the kernel restores that), private
-        to this handle (worker clones run concurrently on other streams and get their own)."""
-        n = 3 * self.ref_shape[0] * self.ref_shape[1]
-        c = self.__dict__.get('_s2_done')
-        if c is None or c.numel() != n or c.device != self.device:
-            c = torch.zeros(n, device=self.device, dtype=torch.int32)
-            self.__dict__['_s2_done'] = c
+    def _s2_counters(self, qn):
+        """Completion counters of the fused S2 kernel for qn queries: zero between calls (the kernel restores
+        that), one buffer per batch size (captured graphs of several sizes keep theirs), private to this handle
+        (worker clones run concurrently on other streams and get their own)."""
+        n = 3 * qn * self.ref_shape[0] * self.ref_shape[1]
+        bufs = self.__dict__.setdefault('_s2_done', {})
+        c = bufs.get(n)
+        if c is None or c.device != self.device:
+            c = bufs[n] = torch.zeros(n, device=self.device, dtype=torch.int32)
         return c
 
     def _finalize(self, ws, rows_total):
@@ -161,36 +163,72 @@ class ViewpointSelector(PackedModule):
         exact, not per-shard."""
         return ops.instnorm_finalize(self.comm.all_reduce_sum(ws), rows_total, IN_EPS)
 
-    def _tower(self, level, ref, scale, shift, cat_buf, S):
-        """corr_conv_list[level] (selector.py:27-69) on the implicit correlation volume."""
-        convs = self.packed()['towers'][level]
-        x, pro, ps, pb = ref, ops.PRO_CORR, scale, shift
-        for i, (pc, post) in enumerate(convs):
-            last = i + 1 == len(convs)
-            if last:
-                ops.conv(x, pc, prologue=pro, pro_scale=ps, pro_shift=pb, group_rows=S, out=cat_buf, out_coff=256 * level)
-                break
-            rows = x.shape[0] * x.shape[1] * x.shape[2]                   # stride-1 same-size convolution
-            y, ws = ops.conv(x, pc, prologue=pro, pro_scale=ps, pro_shift=pb, group_rows=S, stats_rows=rows)
-            # InstanceNorm3d statistics over (S, h, w) of the raw conv output; the normalisation
-            # itself (and the ReLU) is applied by the next conv's loader.  MaxPool commutes with
-            # the positive-slope affine, so pooling the raw tensor first is exact.
-            ps, pb = self._finalize(ws, rows // self.ref_shape[0] * self.rfn_total)
-            pro = ops.PRO_AFFINE_RELU if 'r' in post else ops.PRO_AFFINE
-            x = ops.maxpool2x2(y) if 'p' in post else y
+    # Batched layout: every tensor after the first tower convolution holds qn*S items, query-major (item
+    # g*S + s for query g and reference slice s), so each per-query InstanceNorm group is a run of consecutive
+    # rows and every kernel runs once per batch at M scaled by qn.
 
-    def _towers_sharded(self, q_feats, cat_buf, S, S_total):
+    def _tower_step(self, st, pc, last, cat_buf, level, S, qn):
+        """One convolution of corr_conv_list[level] (selector.py:27-69).  The first reads the shared reference
+        stack (S items) with query g's correlation prologue for output items g*S .. g*S+S-1."""
+        x = st['x']
+        h, w = x.shape[1], x.shape[2]
+        if last:
+            ops.conv(x, pc, prologue=st['pro'], pro_scale=st['ps'], pro_shift=st['pb'], group_rows=S, out=cat_buf,
+                     out_coff=256 * level, batch=qn * S)
+            return None
+        rows = S * h * w                                              # stride-1 same-size convolution: rows per query
+        y, ws = ops.conv(x, pc, prologue=st['pro'], pro_scale=st['ps'], pro_shift=st['pb'], group_rows=S, stats_rows=rows,
+                         batch=qn * S)
+        return y, ws, rows
+
+    def _advance(self, st, post, y, ps, pb):
+        # InstanceNorm3d statistics over (S, h, w) of the raw conv output; the normalisation itself (and the
+        # ReLU) is applied by the next conv's loader.  MaxPool commutes with the positive-slope affine, so
+        # pooling the raw tensor first is exact.
+        st['ps'], st['pb'] = ps, pb
+        st['pro'] = ops.PRO_AFFINE_RELU if 'r' in post else ops.PRO_AFFINE
+        st['x'] = ops.maxpool2x2(y) if 'p' in post else y
+
+    def _tower_states(self, q_feats, S_total):
+        state = []
+        for q, ref, (s1, s2) in zip(q_feats, self.ref_feats_cache, self.ref_sums):
+            qn, h, w, c = q.shape
+            scale, shift = ops.sel_corr_prologue(q.reshape(qn, h * w, c), s1, s2, S_total, IN_EPS)     # one launch per level
+            state.append({'x': ref, 'pro': ops.PRO_CORR, 'ps': scale, 'pb': shift})
+        return state
+
+    def _towers(self, q_feats, cat_buf, S, S_total, qn):
+        """The three towers, each on its own branch stream (they only meet in cat_buf)."""
+        towers = self.packed()['towers']
+        state = self._tower_states(q_feats, S_total)     # prologue launches on the main stream, before the fork
+        br = Branches(3)
+        keep = []
+
+        def run(l, st):
+            convs = towers[l]
+            for i, (pc, post) in enumerate(convs):
+                res = self._tower_step(st, pc, i + 1 == len(convs), cat_buf, l, S, qn)
+                if res is None:
+                    break
+                y, ws, rows = res
+                ps, pb = self._finalize(ws, rows // self.ref_shape[0] * self.rfn_total)
+                self._advance(st, post, y, ps, pb)
+                keep.append(st['x'])
+
+        for l, st in enumerate(state):
+            br.run(l, lambda l=l, st=st: run(l, st))
+        br.join()
+
+    def _towers_sharded(self, q_feats, cat_buf, S, S_total, qn):
         """The three towers with the reference axis sharded over GPUs, ROUND-synchronous: round r runs the
         r-th convolution of every tower that still has one (concurrently, on branch streams), then ONE
-        all-reduce carries the InstanceNorm moments of all of them (5 rounds for the 6 + 4 + 2 convolutions
-        instead of 9 per-layer all-reduces; SURVEY 8e).  Same arithmetic as _tower."""
+        all-reduce carries the InstanceNorm moments [qn, C, 2] of all of them (5 rounds for the 6 + 4 + 2
+        convolutions instead of 9 per-layer all-reduces; SURVEY 8e).  Same arithmetic as _towers."""
         towers = self.packed()['towers']
         nbr = 3 if self.comm.capturable else 1
-        state, keep = [], []
-        for l, (q, ref, (s1, s2)) in enumerate(zip(q_feats, self.ref_feats_cache, self.ref_sums)):
-            h, w, c = q.shape
-            scale, shift = ops.sel_corr_prologue(q.reshape(h * w, c), s1, s2, S_total, IN_EPS)
-            state.append({'x': ref, 'pro': ops.PRO_CORR, 'ps': scale, 'pb': shift, 'i': 0})
+        state, keep = self._tower_states(q_feats, S_total), []
+        for st in state:
+            st['i'] = 0
         for _ in range(max(len(t) for t in towers)):
             br = Branches(nbr)          # forks from the main stream: after the previous round's finalize / pool kernels
             pend = []
@@ -200,16 +238,7 @@ class ViewpointSelector(PackedModule):
                     continue
                 pc, post = convs[st['i']]
                 last = st['i'] + 1 == len(convs)
-
-                def step(l=l, st=st, pc=pc, last=last):
-                    if last:
-                        ops.conv(st['x'], pc, prologue=st['pro'], pro_scale=st['ps'], pro_shift=st['pb'], group_rows=S,
-                                 out=cat_buf, out_coff=256 * l)
-                        return None
-                    rows = st['x'].shape[0] * st['x'].shape[1] * st['x'].shape[2]
-                    return ops.conv(st['x'], pc, prologue=st['pro'], pro_scale=st['ps'], pro_shift=st['pb'], group_rows=S,
-                                    stats_rows=rows) + (rows,)
-                res = br.run(l, step)
+                res = br.run(l, lambda l=l, st=st, pc=pc, last=last: self._tower_step(st, pc, last, cat_buf, l, S, qn))
                 st['i'] += 1
                 if res is not None:
                     pend.append((st, post, res))
@@ -224,90 +253,73 @@ class ViewpointSelector(PackedModule):
                 ps, pb = ops.instnorm_finalize(flat[o:o + n].reshape(ws.shape), rows // self.ref_shape[0] * self.rfn_total, IN_EPS)
                 o += n
                 keep.append((y, ws))
-                st['ps'], st['pb'] = ps, pb
-                st['pro'] = ops.PRO_AFFINE_RELU if 'r' in post else ops.PRO_AFFINE
-                st['x'] = ops.maxpool2x2(y) if 'p' in post else y
+                self._advance(st, post, y, ps, pb)
 
-    def _select_one(self, q_feats):
-        """selector.py:177-215 for one query.  q_feats: 3 x [h, w, 512].  -> logits [rfn], angles [rfn]"""
+    def _select_batch(self, q_feats):
+        """selector.py:177-215 for qn queries in one pass.  q_feats: 3 x [qn, h, w, 512].
+        -> logits [qn, rfn], angles [qn, rfn], scores [qn, 3, S]"""
         p = self.packed()
         rfn, an = self.ref_shape
         S = rfn * an
         S_total = self.rfn_total * an
+        qn = q_feats[0].shape[0]
         dev = self.device
-        cat_buf = torch.empty(S, 4, 4, 768, device=dev, dtype=torch.float32)
-        feats = torch.empty(S, FEAT_PAD, device=dev, dtype=torch.float32)      # cols 0-511: cf3, 512-514 + pad: vp_norm
+        cat_buf = torch.empty(qn * S, 4, 4, 768, device=dev, dtype=torch.float32)
+        feats = torch.empty(qn * S, FEAT_PAD, device=dev, dtype=torch.float32)   # cols 0-511: cf3, 512-514 + pad: vp_norm
         scores = ops.sel_corr_score3([r.reshape(S, -1, r.shape[-1]) for r in self.ref_feats_cache],
-                                     [q.reshape(-1, q.shape[-1]) for q in q_feats], counters=self._s2_counters())
+                                     [q.reshape(qn, -1, q.shape[-1]) for q in q_feats], counters=self._s2_counters(qn))
         if self.comm.world == 1:
-            br = Branches(3)                                # the three towers only meet in cat_buf
-            keep = []
-
-            def one_level(l, q, ref, s1, s2):
-                h, w, c = q.shape
-                scale, shift = ops.sel_corr_prologue(q.reshape(h * w, c), s1, s2, S_total, IN_EPS)
-                keep.append((scale, shift))
-                self._tower(l, ref, scale, shift, cat_buf, S)
-
-            for l, (q, ref, (s1, s2)) in enumerate(zip(q_feats, self.ref_feats_cache, self.ref_sums)):
-                br.run(l, lambda l=l, q=q, ref=ref, s1=s1, s2=s2: one_level(l, q, ref, s1, s2))
-            br.join()
+            self._towers(q_feats, cat_buf, S, S_total, qn)
         else:
-            self._towers_sharded(q_feats, cat_buf, S, S_total)
+            self._towers_sharded(q_feats, cat_buf, S, S_total, qn)
         # corr_feats_conv (selector.py:71-77): 1x1 768->512, IN, ReLU, 1x1 512->512, AvgPool(4,4).
         # The second 1x1 conv is linear, so the 4x4 average is taken first (16x less work).
         y, ws = ops.conv(cat_buf, p['cf0'], stats_rows=S * 16)
         ps, pb = self._finalize(ws, S_total * 16)
-        y = ops.avgpool_affine(y.reshape(S * 16, 512), 16, ps, pb, rows_per_group=S * 16, act=ops.ACT_RELU)
-        ops.conv(y.reshape(S, 1, 1, 512), p['cf3'], out=feats.reshape(S, 1, 1, FEAT_PAD), out_coff=0)
+        y = ops.avgpool_affine(y.reshape(qn * S * 16, 512), 16, ps, pb, rows_per_group=S * 16, act=ops.ACT_RELU)
+        ops.conv(y.reshape(qn * S, 1, 1, 512), p['cf3'], out=feats.reshape(qn * S, 1, 1, FEAT_PAD), out_coff=0)
         if self.comm.world == 1:
             ops.sel_vp_norm(scores, feats, 512, IN_EPS)                 # vp_norm, selector.py:201
-        else:   # InstanceNorm2d over ALL (rfn, an): gather the 3*S_total scores, normalise, keep our rows
-            all_scores = self.comm.all_gather_cat(scores, dim=1).contiguous()
-            tmp = torch.empty(S_total, 4, device=dev, dtype=torch.float32)
+        else:   # InstanceNorm2d over ALL (rfn, an): gather the scores along the slice axis, normalise, keep our rows
+            all_scores = self.comm.all_gather_cat(scores, dim=2).contiguous()
+            tmp = torch.empty(qn * S_total, 4, device=dev, dtype=torch.float32)
             ops.sel_vp_norm(all_scores, tmp, 0, IN_EPS)
             r0, _ = self.comm.shard_range(self.rfn_total)
-            feats[:, 512:516] = tmp[r0 * an:r0 * an + S]
-        x = ops.conv(feats.reshape(S, 1, 1, FEAT_PAD), p['sp0'], act=ops.ACT_RELU)
-        x = ops.conv(x, p['sp2']).reshape(rfn, an, 512)
+            feats.reshape(qn, S, FEAT_PAD)[:, :, 512:516] = tmp.reshape(qn, S_total, 4)[:, r0 * an:r0 * an + S]
+        x = ops.conv(feats.reshape(qn * S, 1, 1, FEAT_PAD), p['sp0'], act=ops.ACT_RELU)
+        x = ops.conv(x, p['sp2']).reshape(qn * rfn, an, 512)
         sf = ops.sel_max_angle_add(x, self.ref_pose_embed)              # selector.py:203-204
         # everything below couples all references (attention, InstanceNorm1d over rfn): gather the
-        # per-reference score features once ([rfn,512] = 128 KB at 64 refs) and run the tail replicated
-        sf = self.comm.all_gather_cat(sf, dim=0).contiguous()
+        # per-reference score features once ([qn, rfn, 512] = 128 KB per query at 64 refs) and run the tail replicated
         rfn_local, rfn = rfn, self.rfn_total
+        if self.comm.world > 1:
+            sf = self.comm.all_gather_cat(sf.reshape(qn, rfn_local, 512), dim=1).reshape(qn * rfn, 512).contiguous()
         for att, (m0, m3) in zip(p['atts'], p['mlps']):
-            x4 = sf.reshape(rfn, 1, 1, 512)
-            qv = ops.conv(x4, att['conv_query']).reshape(rfn, 512)
-            kv = ops.conv(x4, att['conv_key']).reshape(rfn, 512)
-            vv = ops.conv(x4, att['conv_feats']).reshape(rfn, 512)
-            msg = ops.attention(qv, kv, vv, heads=8, head_major=True)
-            msg = ops.conv(msg.reshape(rfn, 1, 1, 512), att['conv_merge']).reshape(rfn, 512)
+            x4 = sf.reshape(qn * rfn, 1, 1, 512)
+            qv = ops.conv(x4, att['conv_query']).reshape(qn * rfn, 512)
+            kv = ops.conv(x4, att['conv_key']).reshape(qn * rfn, 512)
+            vv = ops.conv(x4, att['conv_feats']).reshape(qn * rfn, 512)
+            msg = ops.attention(qv, kv, vv, heads=8, head_major=True, groups=qn)
+            msg = ops.conv(msg.reshape(qn * rfn, 1, 1, 512), att['conv_merge']).reshape(qn * rfn, 512)
             msg = ops.layernorm(msg, att['ln_w'], att['ln_b'], 1e-5)
-            y = ops.conv(torch.cat([sf, msg], 1).reshape(rfn, 1, 1, 1024), m0)
-            ps, pb = ops.instnorm_stats(y, rows_per_group=rfn, eps=IN_EPS)      # InstanceNorm1d over rfn
+            y = ops.conv(torch.cat([sf, msg], 1).reshape(qn * rfn, 1, 1, 1024), m0)
+            ps, pb = ops.instnorm_stats(y, rows_per_group=rfn, eps=IN_EPS)      # InstanceNorm1d over rfn, per query
             y = ops.conv(y, m3, prologue=ops.PRO_AFFINE_RELU, pro_scale=ps, pro_shift=pb, group_rows=rfn)
             ps, pb = ops.instnorm_stats(y, rows_per_group=rfn, eps=IN_EPS)
-            y = ops.affine_act(y.reshape(rfn, 512), ps, pb, rows_per_group=rfn, act=ops.ACT_RELU)
+            y = ops.affine_act(y.reshape(qn * rfn, 512), ps, pb, rows_per_group=rfn, act=ops.ACT_RELU)
             sf = ops.add(y, sf)
-        x = ops.conv(sf.reshape(rfn, 1, 1, 512), p['score_predict'][0], act=ops.ACT_RELU)
-        logits = ops.conv(x, p['score_predict'][1]).reshape(rfn)
-        x = feats.reshape(rfn_local, 1, 1, an * FEAT_PAD)               # angles are per-reference: local
+        x = ops.conv(sf.reshape(qn * rfn, 1, 1, 512), p['score_predict'][0], act=ops.ACT_RELU)
+        logits = ops.conv(x, p['score_predict'][1]).reshape(qn, rfn)
+        x = feats.reshape(qn * rfn_local, 1, 1, an * FEAT_PAD)          # angles are per-reference: local
         for i, pc in enumerate(p['angle_predict']):
             x = ops.conv(x, pc, act=ops.ACT_RELU if i < 2 else ops.ACT_NONE)
-        angles = self.comm.all_gather_cat(x.reshape(rfn_local), dim=0)
+        angles = self.comm.all_gather_cat(x.reshape(qn, rfn_local), dim=1)
         return logits, angles, scores
 
     def _select_nhwc(self, que_norm4):
         if self.ref_feats_cache is None:
             raise RuntimeError('ViewpointSelector: load_ref_imgs / extract_ref_feats must be called first')
-        feats = self._feats(que_norm4)
-        logits, angles, taps = [], [], []
-        for qi in range(que_norm4.shape[0]):
-            lg, ang, sc = self._select_one([f[qi] for f in feats])
-            logits.append(lg)
-            angles.append(ang)
-            taps.append(sc)
-        return torch.stack(logits, 0), torch.stack(angles, 0), torch.stack(taps, 0)
+        return self._select_batch(self._feats(que_norm4))
 
     def _select_u8(self, u8):
         """uint8 crop(s) on the device -> (ref_idx [qn], (angle, logit) [qn,2], logits [qn,rfn])."""

@@ -358,18 +358,24 @@ def transpose_to_packed(x2d):
 
 
 def conv(x, pc, prologue=PRO_NONE, pro_scale=None, pro_shift=None, group_rows=1, act=ACT_NONE,
-         in_coff=0, out=None, out_coff=0, stats_rows=None):
-    """x [B, D, H, W, cs] or [B, H, W, cs]; returns [B, Do, Ho, Wo, Cout] (or 4-D for 4-D input).
+         in_coff=0, out=None, out_coff=0, stats_rows=None, batch=None):
+    """x [B_in, D, H, W, cs] or [B_in, H, W, cs]; returns [B, Do, Ho, Wo, Cout] (or 4-D for 4-D input).
+    batch: output items B (default B_in), a multiple of B_in: output item b reads input item b % B_in (one input
+    stack broadcast to B / B_in prologue groups, e.g. PRO_CORR with scale [B / group_rows, H*W, C]).
+    The prologue group of output item b is b // group_rows.
     stats_rows: also return the InstanceNorm moments of the OUTPUT, (y, ws) with ws float64
     [groups, Cout, 2] = per group of `stats_rows` consecutive output rows (sum y, sum y^2) -- fused into the
     convolution's epilogue on the tensor-core path (no extra pass over y), else by g6d_instnorm_partial;
     pass ws to instnorm_finalize (after any cross-GPU all-reduce)."""
     four = x.dim() == 4
     if four:
-        B, H, W, cs = x.shape
+        B_in, H, W, cs = x.shape
         D = 1
     else:
-        B, D, H, W, cs = x.shape
+        B_in, D, H, W, cs = x.shape
+    B = batch or B_in
+    if B % B_in:
+        raise ValueError(f'conv: batch {B} is not a multiple of the input items {B_in}')
     kd, kh, kw = pc.k
     pd, ph, pw = pc.pad
     s = pc.stride
@@ -379,7 +385,8 @@ def conv(x, pc, prologue=PRO_NONE, pro_scale=None, pro_shift=None, group_rows=1,
         out = torch.empty(shape, device=x.device, dtype=torch.float32)
     d = _lib.ConvDesc(B=B, D=D, H=H, W=W, Cin=pc.cin, in_cstride=cs, in_coff=in_coff, Cout=pc.cout, kd=kd, kh=kh,
                       kw=kw, stride=s, pd=pd, ph=ph, pw=pw, Do=Do, Ho=Ho, Wo=Wo, out_cstride=out.shape[-1],
-                      out_coff=out_coff, prologue=prologue, group_rows=group_rows, act=act, max_chain_k=pc.max_chain_k)
+                      out_coff=out_coff, prologue=prologue, group_rows=group_rows, act=act, max_chain_k=pc.max_chain_k,
+                      in_items=B_in if B != B_in else 0)
     work = 2.0 * B * Do * Ho * Wo * pc.cout * kd * kh * kw * pc.cin
     M = B * Do * Ho * Wo
     stats = None
@@ -482,10 +489,11 @@ def sel_ref_sums(ref):
 
 
 def sel_corr_prologue(q, s1, s2, S, eps=1e-5):
-    Pn, Cc = q.shape
-    scale = torch.empty(Pn, Cc, device=q.device, dtype=torch.float32)
-    shift = torch.empty(Cc, device=q.device, dtype=torch.float32)
-    _call('g6d_sel_corr_prologue', _p(q), _p(s1, torch.float64), _p(s2, torch.float64), S, Pn, Cc, eps, _p(scale),
+    """q [P, C] -> (scale [P, C], shift [C]); or qn queries at once, q [qn, P, C] -> ([qn, P, C], [qn, C])."""
+    qn, Pn, Cc = (1,) + tuple(q.shape) if q.dim() == 2 else q.shape
+    scale = torch.empty(q.shape, device=q.device, dtype=torch.float32)
+    shift = torch.empty(q.shape[:-2] + (Cc,), device=q.device, dtype=torch.float32)
+    _call('g6d_sel_corr_prologue', _p(q), _p(s1, torch.float64), _p(s2, torch.float64), S, Pn, Cc, qn, eps, _p(scale),
           _p(shift), _stream())
     return scale, shift
 
@@ -500,35 +508,47 @@ def sel_corr_score(ref, q, out=None):
 
 
 def sel_corr_score3(refs, qs, counters=None):
-    """refs: 3 x [S, P_l, C]; qs: 3 x [P_l, C] -> score [3, S] in one streaming pass.
-    counters: int32 [3*S], zero (the kernel leaves it zero): one launch; None: dots + finish kernels."""
+    """refs: 3 x [S, P_l, C]; qs: 3 x [P_l, C] -> score [3, S], or qn queries at once, qs: 3 x [qn, P_l, C] ->
+    score [qn, 3, S], in one streaming pass over refs.
+    counters: int32 [3*qn*S], zero (the kernel leaves it zero): one launch; None: dots + finish kernels."""
     S, Cc = refs[0].shape[0], refs[0].shape[2]
     Ps = [r.shape[1] for r in refs]
-    out = torch.empty(3, S, device=refs[0].device, dtype=torch.float32)
-    ws = torch.empty(_lib.lib().g6d_sel_corr_score3_workspace_bytes(S, *Ps) // 4, device=refs[0].device, dtype=torch.float32)
+    qn = 1 if qs[0].dim() == 2 else qs[0].shape[0]
+    out = torch.empty(qs[0].shape[:-2] + (3, S), device=refs[0].device, dtype=torch.float32)
+    ws = torch.empty(_lib.lib().g6d_sel_corr_score3_workspace_bytes(S, *Ps, qn) // 4, device=refs[0].device, dtype=torch.float32)
     _call('g6d_sel_corr_score3', _p(refs[0]), _p(refs[1]), _p(refs[2]), _p(qs[0]), _p(qs[1]), _p(qs[2]), S, Ps[0], Ps[1],
-          Ps[2], Cc, _p(out), _p(ws), _p(counters, torch.int32), _stream(), work=4.0 * (S * sum(Ps) * Cc + sum(Ps) * Cc + 3 * S))
+          Ps[2], Cc, qn, _p(out), _p(ws), _p(counters, torch.int32), _stream(),
+          work=4.0 * (S * sum(Ps) * Cc + qn * (sum(Ps) * Cc + 3 * S)))
     return out
 
 
 def sel_vp_norm(score, feats, coff, eps=1e-5):
-    Ln, n = score.shape
-    _call('g6d_sel_vp_norm', _p(score), Ln, n, eps, _p(feats), feats.shape[-1], coff, _stream())
+    """score [L, n] -> feats rows i; or [groups, L, n] -> feats rows g*n + i (channel coff + l)."""
+    groups, Ln, n = (1,) + tuple(score.shape) if score.dim() == 2 else score.shape
+    _call('g6d_sel_vp_norm', _p(score), groups, Ln, n, eps, _p(feats), feats.shape[-1], coff, _stream())
 
 
 def sel_max_angle_add(x, embed):
-    rfn, an, Cc = x.shape
-    out = torch.empty(rfn, Cc, device=x.device, dtype=torch.float32)
-    _call('g6d_sel_max_angle_add', _p(x), _p(embed), _p(out), rfn, an, Cc, _stream())
+    """x [groups*rfn, an, C], embed [rfn, C] (shared by the groups) -> [groups*rfn, C]."""
+    rows, an, Cc = x.shape
+    rfn = embed.shape[0]
+    if rows % rfn:
+        raise ValueError(f'sel_max_angle_add: {rows} rows are not a whole number of {rfn}-reference groups')
+    out = torch.empty(rows, Cc, device=x.device, dtype=torch.float32)
+    _call('g6d_sel_max_angle_add', _p(x), _p(embed), _p(out), rows // rfn, rfn, an, Cc, _stream())
     return out
 
 
-def attention(q, k, v, heads, head_major=False):
-    """q, k, v [n, C] -> [n, C].  head_major=False: the reference's channel order c = d*heads + head;
+def attention(q, k, v, heads, head_major=False, groups=1):
+    """q, k, v [groups*n, C] -> [groups*n, C]: each group of n consecutive tokens attends within itself.
+    head_major=False: the reference's channel order c = d*heads + head;
     True: c = head*D + d (the tiled kernel; producers / consumer permuted at pack time)."""
-    n, Cc = q.shape
+    rows, Cc = q.shape
+    if rows % groups:
+        raise ValueError(f'attention: {rows} tokens are not {groups} equal groups')
     out = torch.empty_like(q)
-    _call('g6d_attention_headmajor' if head_major else 'g6d_attention', _p(q), _p(k), _p(v), _p(out), n, Cc, heads, _stream())
+    _call('g6d_attention_headmajor' if head_major else 'g6d_attention', _p(q), _p(k), _p(v), _p(out), groups, rows // groups,
+          Cc, heads, _stream())
     return out
 
 

@@ -193,19 +193,22 @@ typedef struct g6d_conv_desc {
     int Do, Ho, Wo;           /* output dims (validated) */
     int out_cstride, out_coff;
     int prologue;             /* G6D_PRO_* applied to in-bounds input elements before the MAC */
-    long long group_rows;     /* G6D_PRO_AFFINE*: input batch items per norm group */
+    long long group_rows;     /* prologue group of output item b: g = b / group_rows */
     int act;                  /* G6D_ACT_* epilogue after bias */
     int max_chain_k;          /* tensor-core path: 0 = default; > 0 bounds the K-elements accumulated into one TMEM
                                  accumulator (longer problems are split and summed in fp32 round-to-nearest).  The tensor
                                  core truncates on every accumulate, which biases long chains of SAME-SIGN products
                                  (detector correlation: post-ReLU features x post-ReLU features) by ~5e-8 per step. */
+    int in_items;             /* input items: 0 = B (item b reads input item b); else a divisor of B and output item b
+                                 reads input item b % in_items (one stack broadcast to B / in_items groups: the batched
+                                 selector's first tower convolution, qn queries against one reference stack) */
 } g6d_conv_desc;
 
 #define G6D_PRO_NONE 0
 #define G6D_PRO_AFFINE 1        /* x*scale[g,c] + shift[g,c]          (folded InstanceNorm)        */
 #define G6D_PRO_AFFINE_RELU 2   /* relu(x*scale[g,c] + shift[g,c])    (folded InstanceNorm + ReLU) */
-#define G6D_PRO_CORR 3          /* x*scale[pos,c] + shift[c]: selector correlation volume
-                                   q (.) ref with the first InstanceNorm3d folded in            */
+#define G6D_PRO_CORR 3          /* x*scale[g,pos,c] + shift[g,c] (scale [groups, D*H*W, Cin], shift [groups, Cin]):
+                                   selector correlation volume q_g (.) ref with the first InstanceNorm3d folded in */
 #define G6D_ACT_NONE 0
 #define G6D_ACT_RELU 1
 #define G6D_ACT_LEAKY01 2
@@ -303,41 +306,45 @@ int g6d_det_parse(const float* scores, const float* scales, const float* offsets
  * [P, C] each.  They give the first InstanceNorm3d's statistics of the correlation volume in
  * closed form at query time (SURVEY.md 8a S2 note). */
 int g6d_sel_ref_sums(const float* ref, int S, int P, int C, double* sum1, double* sum2, g6d_stream_t stream);
-/* From q [P, C] and the sums: scale[p,c] = q[p,c]*rstd_c, shift[c] = -mean_c*rstd_c, the
- * G6D_PRO_CORR prologue operands of the first tower conv (selector.py:28,49,63 InstanceNorm3d
- * over (S,h,w) of que*ref). */
-int g6d_sel_corr_prologue(const float* q, const double* sum1, const double* sum2, int S, int P, int C, float eps,
+/* From the qn queries q [qn, P, C] and the sums: scale[g,p,c] = q[g,p,c]*rstd_gc, shift[g,c] = -mean_gc*rstd_gc,
+ * the G6D_PRO_CORR prologue operands of the first tower conv (selector.py:28,49,63 InstanceNorm3d over (S,h,w)
+ * of que*ref), one launch for all queries. */
+int g6d_sel_corr_prologue(const float* q, const double* sum1, const double* sum2, int S, int P, int C, int qn, float eps,
                           float* scale, float* shift, g6d_stream_t stream);
 /* The rotated-similarity score, selector.py:183-186,192-194: s[p] = sum_c q[p,c]*ref[s,p,c];
  * score[s] = sum_p s[p]^2 / max_p s[p].  ref [S, P, C] is streamed once from HBM. */
 int g6d_sel_corr_score(const float* ref, const float* q, int S, int P, int C, float* score, g6d_stream_t stream);
-/* The same score for the three pyramid levels in one streaming pass (what select_que_imgs uses):
- * score [3, S]; ws: g6d_sel_corr_score3_workspace_bytes(S, P0, P1, P2) bytes (per-location inner
- * products, L2-resident).  counters: 3*S ints, one per (level, slice), ZERO on entry and left zero on
- * exit (allocate + clear once, reuse for every call on the same stream): the CTA that completes the last
- * location of a slice reduces it, so the whole op is one launch.  counters == NULL: two launches. */
-long long g6d_sel_corr_score3_workspace_bytes(int S, int P0, int P1, int P2);
+/* The same score for the three pyramid levels and qn queries in one streaming pass (what select_que_imgs
+ * uses): q_l [qn, P_l, C], score [qn, 3, S]; every reference row is read once and dotted with all qn query
+ * rows (each query's score is bit-identical to a one-query call).  ws: g6d_sel_corr_score3_workspace_bytes(S,
+ * P0, P1, P2, qn) bytes (per-location inner products, L2-resident).  counters: 3*qn*S ints, one per (query,
+ * level, slice), ZERO on entry and left zero on exit (allocate + clear once, reuse for every call on the same
+ * stream): the CTA that completes the last location of a slice reduces it, so the whole op is one launch.
+ * counters == NULL: two launches. */
+long long g6d_sel_corr_score3_workspace_bytes(int S, int P0, int P1, int P2, int qn);
 int g6d_sel_corr_score3(const float* ref0, const float* ref1, const float* ref2, const float* q0, const float* q1,
-                        const float* q2, int S, int P0, int P1, int P2, int C, float* score, float* ws, int* counters,
+                        const float* q2, int S, int P0, int P1, int P2, int C, int qn, float* score, float* ws, int* counters,
                         g6d_stream_t stream);
-/* vp_norm (InstanceNorm2d(3), selector.py:78,201): normalise each of the L score rows [L, n]
- * (biased var, eps) and scatter into feats[n, cstride] at channel coff + l. */
+/* vp_norm (InstanceNorm2d(3), selector.py:78,201) for `groups` queries: normalise each of the L score rows of
+ * score [groups, L, n] (biased var, eps) and scatter into feats[groups * n, cstride] at row g*n + i, channel coff + l. */
 /* (channels [coff + L, cstride) of every feats row -- padding that the consumer multiplies by zero weights -- are set to 0) */
-int g6d_sel_vp_norm(const float* score, int L, int n, float eps, float* feats, int cstride, int coff,
+int g6d_sel_vp_norm(const float* score, int groups, int L, int n, float eps, float* feats, int cstride, int coff,
                     g6d_stream_t stream);
-/* selector.py:203-204: out[r,c] = max_a x[r,a,c] + embed[r,c] */
-int g6d_sel_max_angle_add(const float* x, const float* embed, float* out, int rfn, int an, int C, g6d_stream_t stream);
-/* attention.py:4-17 with the reference's channel->(d, head) mapping c = d*heads + head:
- * q,k,v [n, C] -> out [n, C]; softmax(q_h^T k_h / sqrt(C/heads)) over keys. n <= 1024. */
-int g6d_attention(const float* q, const float* k, const float* v, float* out, int n, int C, int heads,
+/* selector.py:203-204 for `groups` queries: out[g*rfn + r, c] = max_a x[g*rfn + r, a, c] + embed[r, c] */
+int g6d_sel_max_angle_add(const float* x, const float* embed, float* out, int groups, int rfn, int an, int C,
+                          g6d_stream_t stream);
+/* attention.py:4-17 with the reference's channel->(d, head) mapping c = d*heads + head, over `groups`
+ * independent sets of n tokens: q,k,v [groups * n, C] -> out [groups * n, C]; softmax(q_h^T k_h / sqrt(C/heads))
+ * over the keys of the token's own group. n <= 8192. */
+int g6d_attention(const float* q, const float* k, const float* v, float* out, int groups, int n, int C, int heads,
                   g6d_stream_t stream);
 /* The same attention over HEAD-MAJOR channels (c = head*64 + d): the layout a caller gets for free by
  * permuting the output rows of conv_query / conv_key / conv_feats (and the input columns of conv_merge)
  * once at pack time.  Tiled (8 queries x 1 head per block, K / V tiles staged in shared memory by coalesced
  * loads): what the selector uses, and what keeps the replicated tail of a reference-sharded selector
  * (n = all references over all GPUs) cheap.  n <= 2048, C = heads * 64. */
-int g6d_attention_headmajor(const float* q, const float* k, const float* v, float* out, int n, int C, int heads,
-                            g6d_stream_t stream);
+int g6d_attention_headmajor(const float* q, const float* k, const float* v, float* out, int groups, int n, int C,
+                            int heads, g6d_stream_t stream);
 /* nn.LayerNorm(C) over the channel axis of each row (attention.py:19-26) */
 int g6d_layernorm(const float* x, const float* gamma, const float* beta, float* out, int rows, int C, float eps,
                   g6d_stream_t stream);
